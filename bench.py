@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- genomes/hour of the marker-gene search hot path (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 Workloads (config["workload"]):
@@ -24,6 +24,8 @@ plugin: (config 3, N = 1) the drop-in path itself: FASTA files on disk -> Marker
 --impl reference : the CPU arm.  `hmmsearch` itself when it is on PATH (kind "hmmer"); otherwise the CPU restatement of its
         pipeline (oracle/, SSE2 striped MSV/Viterbi filters, every host core; kind "port") followed by the REFERENCE's own
         ResultsParser (oracle/_ref, byte-compiled from /root/reference) -- one full bin x all models per step, no scaling.
+--dump-outputs DIR : after the timed steps, the hit table and QA rows of the last timed step, one .npy per field
+        (dump_outputs).  The workload is generated from fixed seeds, so two builds can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -206,6 +208,32 @@ def total_model_positions(db_path):
     return tot
 
 
+DUMP_BYTES = 60 * 1000 * 1000                 # array data; the .npy headers stay well inside 64 MB
+
+
+def dump_outputs(out_dir, tables, prefix=''):
+    """Writes every field of the structured arrays `tables` ({name: array}) as out_dir/<prefix><name>_<field>.npy: float32
+    fields as float32, all others as float64, with the row indices as <name>_row.npy.  Smallest table first, each takes
+    at most an equal share of what is left of DUMP_BYTES; a table with more rows than that is written as a fixed, seeded
+    sample of its rows, in row order."""
+    os.makedirs(out_dir, exist_ok=True)
+    kinds = {name: {f: (np.float32 if arr.dtype[f].base == np.float32 else np.float64) for f in arr.dtype.names}
+             for name, arr in tables.items()}
+    row_bytes = {name: 8 + sum(np.dtype(k).itemsize * max(1, int(np.prod(tables[name].dtype[f].shape))) for f, k in kinds[name].items())
+                 for name in tables}
+    left = DUMP_BYTES
+    for z, name in enumerate(sorted(tables, key=lambda n: len(tables[n]) * row_bytes[n])):
+        arr = tables[name]
+        cap = left // (len(tables) - z) // row_bytes[name]
+        rows = np.arange(len(arr))
+        if len(arr) > cap:
+            rows = np.sort(np.random.default_rng(0).choice(len(arr), cap, replace=False))
+        left -= len(rows) * row_bytes[name]
+        np.save(os.path.join(out_dir, '%s%s_row.npy' % (prefix, name)), rows.astype(np.float64))
+        for f, kind in kinds[name].items():
+            np.save(os.path.join(out_dir, '%s%s_%s.npy' % (prefix, name, f)), np.ascontiguousarray(arr[f][rows], dtype=kind))
+
+
 def workload_name(cfg, sumM):
     if cfg == 2:
         return "configs[1]: 100 synthetic 2 Mb bins (1,900 ORFs, ~0.59 M residues each) x cpr_43_markers.hmm (43 HMMs, sum M = %d)" % sumM
@@ -374,6 +402,7 @@ def main():
     ap.add_argument('--no-plugin', action='store_true', help='skip the files-on-disk plug-in path measurement')
     ap.add_argument('--profile-plugin', action='store_true', help='cProfile of the plug-in path host code (stderr)')
     ap.add_argument('--pipeline', type=int, default=2, help='batches in flight per GPU (one engine + host thread each)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the hit table and QA rows of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
     if args.impl == 'reference':
         run_reference(args)
@@ -457,11 +486,12 @@ def main():
     def batch_meta(bt):
         if bt.meta is None:
             scaf, num, rank_ = [], [], []
+            scaf_ids = {}                              # the same ids on every run (str hashes change with the process)
             for bi, b in enumerate(bt.bins):
                 order = {n: r for r, n in enumerate(sorted(b.names))}
                 for n in b.names:
                     c = n.rfind('_')
-                    scaf.append(hash((bi, n[:c])) & 0x7fffffff)
+                    scaf.append(scaf_ids.setdefault((bi, n[:c]), len(scaf_ids)))
                     num.append(int(n[c + 1:]))
                     rank_.append(order[n])
             nb = len(bt.bins)
@@ -609,6 +639,10 @@ def main():
     sampler = ClockSampler(local)
     sampler.start()
     recs, t_res, t_res_wall = timed(args.steps, True)
+    if args.dump_outputs:
+        last = recs[-len(step_batches(args.steps - 1)):]      # the batches of the last timed step, in work order
+        dump_outputs(args.dump_outputs, {'hits': np.concatenate([r[0] for r in last]), 'qa': np.concatenate([r[2] for r in last])},
+                     '' if world == 1 else 'rank%d_' % rank)
     ssv_ms = msv_ms = other_ms = 0.0
     launches = cells = pairs = 0
     for hits, st, rows, hm in recs:
@@ -798,7 +832,7 @@ def plugin_path(args, batches, db_path, models):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     t0 = time.perf_counter()
-    n = run('timed', max(args.steps, 2))
+    n = run('timed', args.steps)
     torch.cuda.synchronize()
     ev1.record()
     ev1.synchronize()

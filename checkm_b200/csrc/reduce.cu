@@ -355,9 +355,9 @@ extern "C" int ckm_genome_check(ckm_engine *e, int32_t nbins, const int64_t *bin
 }
 
 
-extern "C" int ckm_reduce(ckm_engine *e, int32_t nmodels_in, int32_t nseq_in, int32_t nbins_in, const ckm_hit *hits, int64_t nhits,
-                          const ckm_reduce_opts *opts, const ckm_reduce_meta *meta,
-                          ckm_qa_row **qa_out, int32_t *nqa_out, ckm_marker_hit **mh_out, int64_t *nmh_out) {
+static int reduce_once(ckm_engine *e, int32_t nmodels_in, int32_t nseq_in, int32_t nbins_in, const ckm_hit *hits, int64_t nhits,
+                       const ckm_reduce_opts *opts, const ckm_reduce_meta *meta,
+                       ckm_qa_row **qa_out, int32_t *nqa_out, ckm_marker_hit **mh_out, int64_t *nmh_out) {
   if (!e || nmodels_in < 0 || nseq_in < 0 || nbins_in < 1 || !opts || !meta || !qa_out || !nqa_out || !mh_out || !nmh_out || (nhits > 0 && !hits)) { set_error("ckm_reduce: bad argument"); return CKM_EINVAL; }
   cudaSetDevice(e->device);
   cudaStream_t st = e->stream;
@@ -464,4 +464,29 @@ extern "C" int ckm_reduce(ckm_engine *e, int32_t nmodels_in, int32_t nseq_in, in
     for (int z = 0; z < mh_len[s]; ++z) out[w++] = mh[(size_t)seg_off[s] + z];
   *qa_out = qa; *nqa_out = nbins; *mh_out = out; *nmh_out = total;
   return CKM_OK;
+}
+
+// Frees what the engine keeps cached between calls: its search workspaces (the next search allocates them again) and the
+// unused blocks of the device's stream-ordered pool.
+static void release_cached_memory(ckm_engine *e) {
+  cudaStreamSynchronize(e->stream);
+  for (auto &s : e->cls) cudaStreamSynchronize(s);
+  if (e->aux) cudaStreamSynchronize(e->aux);
+  for (auto &ent : e->pool) { cudaFree(ent.first); ent = std::make_pair((void *)nullptr, (size_t)0); }
+  cudaMemPool_t mp;
+  if (cudaDeviceGetDefaultMemPool(&mp, e->device) == cudaSuccess) cudaMemPoolTrimTo(mp, 0);
+}
+
+extern "C" int ckm_reduce(ckm_engine *e, int32_t nmodels_in, int32_t nseq_in, int32_t nbins_in, const ckm_hit *hits, int64_t nhits,
+                          const ckm_reduce_opts *opts, const ckm_reduce_meta *meta,
+                          ckm_qa_row **qa_out, int32_t *nqa_out, ckm_marker_hit **mh_out, int64_t *nmh_out) {
+  int rc = reduce_once(e, nmodels_in, nseq_in, nbins_in, hits, nhits, opts, meta, qa_out, nqa_out, mh_out, nmh_out);
+  if (rc == CKM_ENOMEM) {
+    // after a large search the engine's cached workspaces can hold most of the device: a reduction over many bins
+    // (one analyseResults over a whole directory) then finds no room for its rows
+    cudaGetLastError();              // the failed allocation must not surface as a launch error of the retry
+    release_cached_memory(e);
+    rc = reduce_once(e, nmodels_in, nseq_in, nbins_in, hits, nhits, opts, meta, qa_out, nqa_out, mh_out, nmh_out);
+  }
+  return rc;
 }

@@ -226,7 +226,9 @@ typedef struct {
 } ckm_reduce_meta;
 
 /* hits: domtblout rows grouped by bin (ascending) and, inside a bin, by query (rows of one query contiguous, in file
- * order).  `model` and `seq` index the caller's model table (nmodels entries) and sequence table (nseq entries). */
+ * order).  `model` and `seq` index the caller's model table (nmodels entries) and sequence table (nseq entries).
+ * When the device has no room left for the reduction, the engine's cached search workspaces are freed and the call is
+ * tried once more; the engine's next search allocates them again. */
 int  ckm_reduce(ckm_engine *e, int32_t nmodels, int32_t nseq, int32_t nbins, const ckm_hit *hits, int64_t nhits,
                 const ckm_reduce_opts *opts, const ckm_reduce_meta *meta,
                 ckm_qa_row **qa_out, int32_t *nqa_out, ckm_marker_hit **mh_out, int64_t *nmh_out);
