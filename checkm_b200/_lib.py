@@ -66,7 +66,7 @@ class ReduceMeta(C.Structure):
 SYMBOLS = ["ckm_init", "ckm_destroy", "ckm_last_error", "ckm_version", "ckm_device_name",
            "ckm_models_load", "ckm_models_count", "ckm_models_info", "ckm_models_find", "ckm_models_select",
            "ckm_models_write", "ckm_models_free", "ckm_digitize", "ckm_fasta_parse", "ckm_seqdb_create", "ckm_seqdb_free",
-           "ckm_search", "ckm_search_per_bin", "ckm_hits_free", "ckm_align", "ckm_last_stats", "ckm_msv_scores",
+           "ckm_search", "ckm_search_per_bin", "ckm_hits_free", "ckm_align", "ckm_last_stats", "ckm_workspace_bytes", "ckm_msv_scores",
            "ckm_filter_scores", "ckm_viterbi_scores", "ckm_write_domtblout", "ckm_reduce", "ckm_genome_check", "ckm_free", "ckm_allgather_qa", "ckm_nccl_unique_id",
            "ckm_nccl_comm_init", "ckm_nccl_comm_destroy", "ckm_fasta_scan_nt", "ckm_scaffold_stats"]
 
@@ -109,6 +109,7 @@ def lib():
     L.ckm_hits_free.argtypes = [C.POINTER(Hit)]
     L.ckm_hits_free.restype = None
     L.ckm_last_stats.argtypes = [vp, C.POINTER(Stats)]
+    L.ckm_workspace_bytes.argtypes = [vp, C.POINTER(i64)]
     L.ckm_msv_scores.argtypes = [vp, vp, vp, i32, vp, vp]
     L.ckm_filter_scores.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp, vp]
     L.ckm_viterbi_scores.argtypes = [vp, vp, vp, i32, vp, i32, vp]

@@ -8,6 +8,7 @@
 #include <stdexcept>
 #include <atomic>
 #include "engine.hpp"
+#include "pool.hpp"
 
 namespace ckm {
 const std::string &get_error();
@@ -75,8 +76,7 @@ void ckm_destroy(ckm_engine *e) {
   for (auto &ev : e->cls_ev) cudaEventDestroy(ev);
   cudaEventDestroy(e->fan_ev);
   cudaFree(e->d_counters);
-  cudaFree(e->d_scratch);
-  for (auto &ent : e->pool) cudaFree(ent.first);
+  workspace_release(e);
   cudaStreamDestroy(e->stream);
   delete e;
 }
@@ -317,6 +317,13 @@ void ckm_hits_free(ckm_hit *hits) { std::free(hits); }
 int ckm_last_stats(const ckm_engine *e, ckm_stats *out) {
   if (!e || !out) { set_error("ckm_last_stats: bad argument"); return CKM_EINVAL; }
   *out = e->stats;
+  return CKM_OK;
+}
+
+int ckm_workspace_bytes(const ckm_engine *e, int64_t *bytes_out) {
+  if (!e || !bytes_out) { set_error("ckm_workspace_bytes: bad argument"); return CKM_EINVAL; }
+  *bytes_out = 0;
+  for (const auto &w : e->ws) *bytes_out += (int64_t)w.bytes;
   return CKM_OK;
 }
 

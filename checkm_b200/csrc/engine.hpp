@@ -78,6 +78,20 @@ struct Candidate {       // an (ORF, HMM) pair moving down the cascade
   double  P;             // P-value after the latest stage
 };
 
+// Workspace roles: each keys one grow-only device buffer of the engine (pool.hpp).  Buffers that are live at the same time in
+// one call never share a key.  Shared between entry points (same role; one engine runs one call at a time): the filter-cascade
+// keys by every entry point that runs the cascade, and Pairs, Vec, Doms, EnvScratch, Envs1, EnvOrder1 by search and alignment.
+enum class Ws : int {
+  ModelSlot, ModelActive, TileActive, Cand, Pass, Cells, Bnd, GroupList, ListA, ListB, Redo,
+  SlotModel, DenseFiltersc, DenseVit, DenseFwd, DensePassed, DenseXj,
+  Pairs, Xf, Xb, Vec, LogsumTbl, Regions, PairOrder, Doms, Hits, AlignTrace,
+  EnvScratch, Envs1, EnvOrder1, Envs2, EnvOrder2,
+  EnsRegions, EnsMultiIdx, EnsScratchOff, EnsScratch, EnsEnvs, EnsCount, EnsCaps, EnsEnvOff, EnsNeed,   // the trace ensemble (on `aux`)
+  NtBytes, NtRows, NtPieces, NtStats, NtContigScaf, NtContigLen, NtCounters,
+  Gather,
+  Count
+};
+
 }  // namespace ckm
 
 // ------------------------------------------------------------------------------------------------
@@ -159,9 +173,8 @@ struct ckm_engine {
   cudaEvent_t cls_ev[NCLS], fan_ev;
   cudaStream_t aux = nullptr;     // the trace-ensemble job of a search runs here, next to the class streams
   ckm_stats stats;
-  // grow-only device buffer cache: slot -> (pointer, bytes); search/reduce workspaces are reused across calls
-  std::vector<std::pair<void *, size_t>> pool;
-  void   *d_scratch = nullptr; size_t scratch_bytes = 0;
+  // device workspaces by role, reused by every later call (pool.hpp)
+  struct { void *p = nullptr; size_t bytes = 0; } ws[(int)ckm::Ws::Count];
   int32_t *d_counters = nullptr;   // small array of device counters
 };
 

@@ -6,6 +6,7 @@
 #include <mutex>
 #include <vector>
 #include "engine.hpp"
+#include "pool.hpp"
 
 using namespace ckm;
 
@@ -89,13 +90,9 @@ int ckm_allgather_qa(ckm_engine *e, void *nccl_comm, const ckm_qa_row *rows, int
   CKM_CUDA(cudaSetDevice(e->device));
   const size_t slot = 8 + (size_t)nrows_max * sizeof(ckm_qa_row);
   const size_t need = slot * ((size_t)world + 1);
-  if (e->scratch_bytes < need) {
-    if (e->d_scratch) cudaFree(e->d_scratch);
-    e->d_scratch = nullptr; e->scratch_bytes = 0;
-    CKM_CUDA(cudaMalloc(&e->d_scratch, need));
-    e->scratch_bytes = need;
-  }
-  uint8_t *d_send = (uint8_t *)e->d_scratch, *d_recv = d_send + slot;
+  uint8_t *d_send;
+  if ((rc = workspace(e, Ws::Gather, need, &d_send))) return rc;
+  uint8_t *d_recv = d_send + slot;
   std::vector<uint8_t> host(slot * (size_t)world, 0);
   const int64_t cnt = nrows;
   std::memcpy(host.data(), &cnt, 8);

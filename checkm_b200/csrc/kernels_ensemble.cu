@@ -405,7 +405,6 @@ __global__ void __launch_bounds__(FWD_WARPS * 32) ensemble_kernel(EnsembleParams
 // The ensemble of all multi-domain regions as an asynchronous job on stream `st`: ensembles_launch enqueues the uploads,
 // the kernel and the downloads; ensembles_collect waits for them and hands back the envelopes of every region.
 struct EnsembleJob {
-  DevBuf b_regs, b_idx, b_off, b_scr, b_env, b_cnt, b_caps, b_eoff, b_need;       // workspaces from the engine's cache (the caller holds the PoolScope)
   std::vector<int64_t> off, env_off;
   std::vector<Envelope> envs;
   std::vector<int32_t> cnt, need;
@@ -430,22 +429,26 @@ int ensembles_launch(ckm_engine *e, const ckm_models *m, DomdefParams &p, const 
     job->env_off[i] = nenv;
     nenv += caps[i].envelopes;
   }
+  // its own keys: the envelope waves run next to it on the class streams
+  Region *regs_d; int32_t *idx_d, *cnt_d, *need_d; int64_t *off_d, *eoff_d; float *scr_d; Envelope *env_d; EnsembleCaps *caps_d;
   int rc;
-  if ((rc = job->b_regs.alloc(sizeof(Region) * regs.size())) || (rc = job->b_idx.alloc(sizeof(int32_t) * nm)) || (rc = job->b_off.alloc(sizeof(int64_t) * nm)) ||
-      (rc = job->b_scr.alloc(sizeof(float) * (size_t)tot)) || (rc = job->b_env.alloc(sizeof(Envelope) * (size_t)nenv)) || (rc = job->b_cnt.alloc(sizeof(int32_t) * nm)) ||
-      (rc = job->b_caps.alloc(sizeof(EnsembleCaps) * nm)) || (rc = job->b_eoff.alloc(sizeof(int64_t) * nm)) || (rc = job->b_need.alloc(sizeof(int32_t) * 3 * nm))) return rc;
-  CKM_CUDA(cudaMemcpyAsync(job->b_regs.p, regs.data(), sizeof(Region) * regs.size(), cudaMemcpyHostToDevice, st));       // regs, multi_idx outlive the job (caller)
-  CKM_CUDA(cudaMemcpyAsync(job->b_idx.p, multi_idx.data(), sizeof(int32_t) * nm, cudaMemcpyHostToDevice, st));
-  CKM_CUDA(cudaMemcpyAsync(job->b_off.p, job->off.data(), sizeof(int64_t) * nm, cudaMemcpyHostToDevice, st));
-  CKM_CUDA(cudaMemcpyAsync(job->b_caps.p, job->caps.data(), sizeof(EnsembleCaps) * nm, cudaMemcpyHostToDevice, st));
-  CKM_CUDA(cudaMemcpyAsync(job->b_eoff.p, job->env_off.data(), sizeof(int64_t) * nm, cudaMemcpyHostToDevice, st));
-  CKM_CUDA(cudaMemsetAsync(job->b_cnt.p, 0, sizeof(int32_t) * nm, st));
-  CKM_CUDA(cudaMemsetAsync(job->b_need.p, 0, sizeof(int32_t) * 3 * nm, st));
-  CKM_CUDA(cudaMemsetAsync(job->b_env.p, 0, sizeof(Envelope) * (size_t)nenv, st));      // the kernel fills only the slots it uses; the whole block is copied back
+  if ((rc = workspace(e, Ws::EnsRegions, sizeof(Region) * regs.size(), &regs_d)) || (rc = workspace(e, Ws::EnsMultiIdx, sizeof(int32_t) * nm, &idx_d)) ||
+      (rc = workspace(e, Ws::EnsScratchOff, sizeof(int64_t) * nm, &off_d)) || (rc = workspace(e, Ws::EnsScratch, sizeof(float) * (size_t)tot, &scr_d)) ||
+      (rc = workspace(e, Ws::EnsEnvs, sizeof(Envelope) * (size_t)nenv, &env_d)) || (rc = workspace(e, Ws::EnsCount, sizeof(int32_t) * nm, &cnt_d)) ||
+      (rc = workspace(e, Ws::EnsCaps, sizeof(EnsembleCaps) * nm, &caps_d)) || (rc = workspace(e, Ws::EnsEnvOff, sizeof(int64_t) * nm, &eoff_d)) ||
+      (rc = workspace(e, Ws::EnsNeed, sizeof(int32_t) * 3 * nm, &need_d))) return rc;
+  CKM_CUDA(cudaMemcpyAsync(regs_d, regs.data(), sizeof(Region) * regs.size(), cudaMemcpyHostToDevice, st));       // regs, multi_idx outlive the job (caller)
+  CKM_CUDA(cudaMemcpyAsync(idx_d, multi_idx.data(), sizeof(int32_t) * nm, cudaMemcpyHostToDevice, st));
+  CKM_CUDA(cudaMemcpyAsync(off_d, job->off.data(), sizeof(int64_t) * nm, cudaMemcpyHostToDevice, st));
+  CKM_CUDA(cudaMemcpyAsync(caps_d, job->caps.data(), sizeof(EnsembleCaps) * nm, cudaMemcpyHostToDevice, st));
+  CKM_CUDA(cudaMemcpyAsync(eoff_d, job->env_off.data(), sizeof(int64_t) * nm, cudaMemcpyHostToDevice, st));
+  CKM_CUDA(cudaMemsetAsync(cnt_d, 0, sizeof(int32_t) * nm, st));
+  CKM_CUDA(cudaMemsetAsync(need_d, 0, sizeof(int32_t) * 3 * nm, st));
+  CKM_CUDA(cudaMemsetAsync(env_d, 0, sizeof(Envelope) * (size_t)nenv, st));      // the kernel fills only the slots it uses; the whole block is copied back
   EnsembleParams ep;
-  ep.d = p; ep.regions = job->b_regs.as<Region>(); ep.multi_idx = job->b_idx.as<int32_t>(); ep.nmulti = nm;
-  ep.scratch_off = job->b_off.as<int64_t>(); ep.scratch = job->b_scr.as<float>(); ep.env_out = job->b_env.as<Envelope>(); ep.env_count = job->b_cnt.as<int32_t>();
-  ep.caps = job->b_caps.as<EnsembleCaps>(); ep.env_off = job->b_eoff.as<int64_t>(); ep.need = job->b_need.as<int32_t>();
+  ep.d = p; ep.regions = regs_d; ep.multi_idx = idx_d; ep.nmulti = nm;
+  ep.scratch_off = off_d; ep.scratch = scr_d; ep.env_out = env_d; ep.env_count = cnt_d;
+  ep.caps = caps_d; ep.env_off = eoff_d; ep.need = need_d;
   const size_t smem = (size_t)FWD_WARPS * 3 * p.row_elems * sizeof(float);
   CKM_CUDA(cudaFuncSetAttribute(ensemble_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int grid = std::min(e->prop.multiProcessorCount * 4, (nm + FWD_WARPS - 1) / FWD_WARPS);
@@ -454,9 +457,9 @@ int ensembles_launch(ckm_engine *e, const ckm_models *m, DomdefParams &p, const 
   e->stats.kernel_launches++;
   job->envs.resize((size_t)nenv);
   job->cnt.resize(nm); job->need.resize((size_t)3 * nm);
-  CKM_CUDA(cudaMemcpyAsync(job->envs.data(), job->b_env.p, sizeof(Envelope) * job->envs.size(), cudaMemcpyDeviceToHost, st));
-  CKM_CUDA(cudaMemcpyAsync(job->cnt.data(), job->b_cnt.p, sizeof(int32_t) * nm, cudaMemcpyDeviceToHost, st));
-  CKM_CUDA(cudaMemcpyAsync(job->need.data(), job->b_need.p, sizeof(int32_t) * 3 * nm, cudaMemcpyDeviceToHost, st));
+  CKM_CUDA(cudaMemcpyAsync(job->envs.data(), env_d, sizeof(Envelope) * job->envs.size(), cudaMemcpyDeviceToHost, st));
+  CKM_CUDA(cudaMemcpyAsync(job->cnt.data(), cnt_d, sizeof(int32_t) * nm, cudaMemcpyDeviceToHost, st));
+  CKM_CUDA(cudaMemcpyAsync(job->need.data(), need_d, sizeof(int32_t) * 3 * nm, cudaMemcpyDeviceToHost, st));
   return CKM_OK;
 }
 

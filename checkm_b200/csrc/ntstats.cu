@@ -339,10 +339,10 @@ int ckm_scaffold_stats(ckm_engine *e, const uint8_t *bytes, int64_t nbytes, cons
     }
   }
   cudaSetDevice(e->device);
-  PoolScope pool_scope(e);
   cudaStream_t st = e->stream;
-  DevBuf dbytes;
-  { int rc0 = dbytes.alloc((size_t)nbytes + 64); if (rc0) return rc0; }
+  uint8_t *dbytes;
+  int rc;
+  if ((rc = workspace(e, Ws::NtBytes, (size_t)nbytes + 64, &dbytes))) return rc;
   std::vector<NtRow> rows;
   rows.reserve((size_t)(nbytes / NT_ROW) + nscaf);
   for (int32_t s = 0; s < nscaf; ++s)
@@ -350,7 +350,7 @@ int ckm_scaffold_stats(ckm_engine *e, const uint8_t *bytes, int64_t nbytes, cons
       const int64_t n = std::min<int64_t>(NT_ROW, lens[s] - off);
       const bool first = off == 0, last = off + NT_ROW >= lens[s];
       const int64_t left = first ? 0 : NT_HALO, copy = left + (n + 63) / 64 * 64 + (last ? 0 : NT_HALO);
-      NtRow r; r.src = (uint64_t)(uintptr_t)(dbytes.as<uint8_t>() + starts[s] + off - left); r.scaf = (uint32_t)s;
+      NtRow r; r.src = (uint64_t)(uintptr_t)(dbytes + starts[s] + off - left); r.scaf = (uint32_t)s;
       r.info = (uint32_t)n | ((uint32_t)(copy / 16) << 12) | (first ? 1u << 30 : 0u) | (last ? 1u << 31 : 0u);
       rows.push_back(r);
     }
@@ -361,22 +361,20 @@ int ckm_scaffold_stats(ckm_engine *e, const uint8_t *bytes, int64_t nbytes, cons
   const int grid = (int)std::min<int64_t>((int64_t)e->prop.multiProcessorCount * NT_CTAS_PER_SM, (nrows + NT_WARPS - 1) / NT_WARPS);
   const int64_t nwarps = (int64_t)grid * NT_WARPS;
   const size_t npiece = (size_t)nscaf + nwarps;
-  DevBuf drows, dpiece, dstats, dcs, dcl, dctr;
-  int rc;
-  if ((rc = drows.alloc(sizeof(NtRow) * nrows)) || (rc = dpiece.alloc(sizeof(NtPiece) * npiece)) ||
-      (rc = dstats.alloc(sizeof(int64_t) * 8 * nscaf)) ||
-      (rc = dcs.alloc(sizeof(uint32_t) * (size_t)contig_cap)) || (rc = dcl.alloc(sizeof(uint32_t) * (size_t)contig_cap)) || (rc = dctr.alloc(64)))
-    return rc;
-  CKM_CUDA(cudaMemcpyAsync(dbytes.p, bytes, (size_t)nbytes, cudaMemcpyHostToDevice, st));
-  CKM_CUDA(cudaMemcpyAsync(drows.p, rows.data(), sizeof(NtRow) * nrows, cudaMemcpyHostToDevice, st));
-  CKM_CUDA(cudaMemsetAsync(dpiece.p, 0, sizeof(NtPiece) * npiece, st));
-  CKM_CUDA(cudaMemsetAsync(dctr.p, 0, 64, st));
-  CKM_CUDA(cudaMemsetAsync(dstats.p, 0, sizeof(int64_t) * 8 * nscaf, st));
   NtParams p;
-  p.bytes = dbytes.as<uint8_t>(); p.rows = drows.as<NtRow>(); p.nrows = nrows; p.piece = dpiece.as<NtPiece>();
-  p.stats = dstats.as<unsigned long long>();
-  p.contig_scaf = dcs.as<uint32_t>(); p.contig_len = dcl.as<uint32_t>();
-  p.ncontigs = reinterpret_cast<unsigned long long *>(dctr.as<uint8_t>() + 8); p.cap = contig_cap;
+  NtRow *drows; uint8_t *dctr;
+  if ((rc = workspace(e, Ws::NtRows, sizeof(NtRow) * nrows, &drows)) || (rc = workspace(e, Ws::NtPieces, sizeof(NtPiece) * npiece, &p.piece)) ||
+      (rc = workspace(e, Ws::NtStats, sizeof(int64_t) * 8 * nscaf, &p.stats)) ||
+      (rc = workspace(e, Ws::NtContigScaf, sizeof(uint32_t) * (size_t)contig_cap, &p.contig_scaf)) ||
+      (rc = workspace(e, Ws::NtContigLen, sizeof(uint32_t) * (size_t)contig_cap, &p.contig_len)) || (rc = workspace(e, Ws::NtCounters, 64, &dctr)))
+    return rc;
+  CKM_CUDA(cudaMemcpyAsync(dbytes, bytes, (size_t)nbytes, cudaMemcpyHostToDevice, st));
+  CKM_CUDA(cudaMemcpyAsync(drows, rows.data(), sizeof(NtRow) * nrows, cudaMemcpyHostToDevice, st));
+  CKM_CUDA(cudaMemsetAsync(p.piece, 0, sizeof(NtPiece) * npiece, st));
+  CKM_CUDA(cudaMemsetAsync(dctr, 0, 64, st));
+  CKM_CUDA(cudaMemsetAsync(p.stats, 0, sizeof(int64_t) * 8 * nscaf, st));
+  p.bytes = dbytes; p.rows = drows; p.nrows = nrows;
+  p.ncontigs = reinterpret_cast<unsigned long long *>(dctr + 8); p.cap = contig_cap;
   const int dyn_smem = NT_WARPS * NT_WARP_SMEM;
   CKM_CUDA(cudaFuncSetAttribute(ntstats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_smem));
   CKM_CUDA(cudaEventRecord(e->ev[0], st));
@@ -386,8 +384,8 @@ int ckm_scaffold_stats(ckm_engine *e, const uint8_t *bytes, int64_t nbytes, cons
   unsigned long long n_dev = 0;
   std::vector<NtPiece> piece(npiece);
   CKM_CUDA(cudaMemcpyAsync(&n_dev, p.ncontigs, sizeof(n_dev), cudaMemcpyDeviceToHost, st));
-  CKM_CUDA(cudaMemcpyAsync(stats_out, dstats.p, sizeof(int64_t) * 8 * nscaf, cudaMemcpyDeviceToHost, st));
-  CKM_CUDA(cudaMemcpyAsync(piece.data(), dpiece.p, sizeof(NtPiece) * npiece, cudaMemcpyDeviceToHost, st));
+  CKM_CUDA(cudaMemcpyAsync(stats_out, p.stats, sizeof(int64_t) * 8 * nscaf, cudaMemcpyDeviceToHost, st));
+  CKM_CUDA(cudaMemcpyAsync(piece.data(), p.piece, sizeof(NtPiece) * npiece, cudaMemcpyDeviceToHost, st));
   CKM_CUDA(cudaStreamSynchronize(st));
   if (kernel_ms_out) CKM_CUDA(cudaEventElapsedTime(kernel_ms_out, e->ev[0], e->ev[1]));
   // join the open ends of the pieces, in list order: a contig runs from the tail of one piece through every piece without a
@@ -412,8 +410,8 @@ int ckm_scaffold_stats(ckm_engine *e, const uint8_t *bytes, int64_t nbytes, cons
   *ncontigs_out = n_found;
   if (n_found > contig_cap) { set_error("ckm_scaffold_stats: more contigs than the caller allowed for (the count is returned; call again)"); return CKM_ECAPACITY; }
   if (n_dev) {
-    CKM_CUDA(cudaMemcpyAsync(contig_scaffold_out, dcs.p, sizeof(uint32_t) * n_dev, cudaMemcpyDeviceToHost, st));
-    CKM_CUDA(cudaMemcpyAsync(contig_len_out, dcl.p, sizeof(uint32_t) * n_dev, cudaMemcpyDeviceToHost, st));
+    CKM_CUDA(cudaMemcpyAsync(contig_scaffold_out, p.contig_scaf, sizeof(uint32_t) * n_dev, cudaMemcpyDeviceToHost, st));
+    CKM_CUDA(cudaMemcpyAsync(contig_len_out, p.contig_len, sizeof(uint32_t) * n_dev, cudaMemcpyDeviceToHost, st));
     CKM_CUDA(cudaStreamSynchronize(st));
   }
   for (size_t k = 0; k < joined.size(); ++k) {

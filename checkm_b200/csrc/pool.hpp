@@ -1,37 +1,33 @@
-// pool.hpp -- workspace buffers handed out from the engine's grow-only device cache
+// pool.hpp -- the engine's workspace table: one grow-only device buffer per role (ckm::Ws), reused by every later call
 #pragma once
 #include <algorithm>
 #include "engine.hpp"
 
 namespace ckm {
 
-// ---- device buffers come from the engine's grow-only cache: no cudaMalloc/cudaFree in the steady state ----
-extern thread_local ckm_engine *g_pool_engine;   // one search per host thread; engines are not shared between threads (defined in search.cu)
-extern thread_local int g_pool_next;
-struct PoolScope {           // every search starts handing out slots from 0 again
-  explicit PoolScope(ckm_engine *e) { g_pool_engine = e; g_pool_next = 0; }
-  ~PoolScope() { g_pool_engine = nullptr; }
-};
-struct DevBuf {
-  void *p = nullptr; size_t bytes = 0; int slot = -1;
-  int alloc(size_t n) {
-    ckm_engine *e = g_pool_engine;
-    if (e == nullptr) { set_error("internal: workspace requested outside a search"); return CKM_EINVAL; }
-    if (slot < 0) { slot = g_pool_next++; if ((size_t)slot >= e->pool.size()) e->pool.resize(slot + 1, std::make_pair((void *)nullptr, (size_t)0)); }
-    bytes = std::max<size_t>(n, 256);
-    auto &ent = e->pool[slot];
-    if (ent.second < bytes) {
-      if (ent.first) cudaFree(ent.first);
-      ent.first = nullptr; ent.second = 0;
-      const size_t want = bytes + bytes / 4;
-      cudaError_t err = cudaMalloc(&ent.first, want);
-      if (err != cudaSuccess) { err = cudaMalloc(&ent.first, bytes); if (err != cudaSuccess) { ent.first = nullptr; p = nullptr; return cuda_fail(err, "cudaMalloc(workspace)"); } ent.second = bytes; }
-      else ent.second = want;
+// The engine's buffer for `key`, at least `bytes` (and 256) long.  A buffer that is too small is freed and allocated again with
+// 25% slack, or exactly `bytes` when the slack does not fit; its contents are not kept.
+template <class T> int workspace(ckm_engine *e, Ws key, size_t bytes, T **out) {
+  auto &w = e->ws[(int)key];
+  bytes = std::max<size_t>(bytes, 256);
+  if (w.bytes < bytes) {
+    cudaFree(w.p);
+    w.p = nullptr; w.bytes = 0;
+    const size_t want = bytes + bytes / 4;
+    if (cudaMalloc(&w.p, want) == cudaSuccess) w.bytes = want;
+    else {
+      const cudaError_t err = cudaMalloc(&w.p, bytes);
+      if (err != cudaSuccess) { w.p = nullptr; *out = nullptr; return cuda_fail(err, "cudaMalloc(workspace)"); }
+      w.bytes = bytes;
     }
-    p = ent.first;
-    return CKM_OK;
   }
-  template <class T> T *as() { return reinterpret_cast<T *>(p); }
-};
+  *out = static_cast<T *>(w.p);
+  return CKM_OK;
+}
+
+// Frees every workspace (the next call allocates what it needs again).  No stream of the engine may still use them.
+inline void workspace_release(ckm_engine *e) {
+  for (auto &w : e->ws) { cudaFree(w.p); w.p = nullptr; w.bytes = 0; }
+}
 
 }  // namespace ckm

@@ -12,6 +12,7 @@
 #include <cstring>
 #include <vector>
 #include "engine.hpp"
+#include "pool.hpp"
 
 namespace ckm {
 
@@ -324,6 +325,28 @@ __global__ void genome_check_kernel(int32_t nbins, const int64_t *bin_set_off, c
   }
 }
 
+// Device buffers of one call, from the stream-ordered pool (none of them stays resident), handed back to it stream-ordered (no
+// device-wide synchronisation) when the holder goes out of scope.
+struct CallBuffers {
+  cudaStream_t st; const char *who;
+  std::vector<void *> held;
+  CallBuffers(cudaStream_t s, const char *w) : st(s), who(w) {}
+  CallBuffers(const CallBuffers &) = delete;
+  ~CallBuffers() { for (void *q : held) cudaFreeAsync(q, st); }
+  // n elements (at least 16 bytes); CKM_ENOMEM when the device has no room.  upload: filled from the host.
+  template <class T> int get(T **out, size_t n) {
+    void *q = nullptr;
+    if (cudaMallocAsync(&q, std::max<size_t>(sizeof(T) * n, 16), st) != cudaSuccess) { set_error(std::string(who) + ": out of device memory"); return CKM_ENOMEM; }
+    held.push_back(q); *out = static_cast<T *>(q);
+    return CKM_OK;
+  }
+  template <class T> int upload(T **out, const void *src, size_t n) {
+    const int rc = get(out, n);
+    if (rc == CKM_OK && n > 0) CKM_CUDA(cudaMemcpyAsync((void *)*out, src, sizeof(T) * n, cudaMemcpyHostToDevice, st));
+    return rc;
+  }
+};
+
 }  // namespace ckm
 
 using namespace ckm;
@@ -335,21 +358,15 @@ extern "C" int ckm_genome_check(ckm_engine *e, int32_t nbins, const int64_t *bin
   cudaSetDevice(e->device);
   cudaStream_t st = e->stream;
   const int64_t nsets = bin_set_off[nbins], nm = set_marker_off[nsets];
-  void *d_b = nullptr, *d_s = nullptr, *d_c = nullptr, *d_o = nullptr;
-  auto cleanup = [&]() { for (void *q : {d_b, d_s, d_c, d_o}) if (q) cudaFreeAsync(q, st); };       // stream-ordered pool: no device-wide synchronisation
-#define GCUDA(call) do { cudaError_t _e = (call); if (_e != cudaSuccess) { cleanup(); return cuda_fail(_e, #call); } } while (0)
-  GCUDA(cudaMallocAsync(&d_b, sizeof(int64_t) * (nbins + 1), st));
-  GCUDA(cudaMallocAsync(&d_s, sizeof(int64_t) * (size_t)(nsets + 1), st));
-  GCUDA(cudaMallocAsync(&d_c, sizeof(int32_t) * (size_t)std::max<int64_t>(nm, 1), st));
-  GCUDA(cudaMallocAsync(&d_o, sizeof(ckm_qa_row) * nbins, st));
-  GCUDA(cudaMemcpyAsync(d_b, bin_set_off, sizeof(int64_t) * (nbins + 1), cudaMemcpyHostToDevice, st));
-  GCUDA(cudaMemcpyAsync(d_s, set_marker_off, sizeof(int64_t) * (size_t)(nsets + 1), cudaMemcpyHostToDevice, st));
-  if (nm > 0) GCUDA(cudaMemcpyAsync(d_c, marker_count, sizeof(int32_t) * (size_t)nm, cudaMemcpyHostToDevice, st));
-  genome_check_kernel<<<(nbins + 127) / 128, 128, 0, st>>>(nbins, (const int64_t *)d_b, (const int64_t *)d_s, (const int32_t *)d_c, individual_markers, (ckm_qa_row *)d_o);
-  GCUDA(cudaGetLastError());
-  GCUDA(cudaMemcpyAsync(rows_out, d_o, sizeof(ckm_qa_row) * nbins, cudaMemcpyDeviceToHost, st));
-  GCUDA(cudaStreamSynchronize(st));
-  cleanup();
+  CallBuffers mem(st, "ckm_genome_check");
+  int64_t *d_b, *d_s; int32_t *d_c; ckm_qa_row *d_o;
+  int rc;
+  if ((rc = mem.upload(&d_b, bin_set_off, (size_t)nbins + 1)) || (rc = mem.upload(&d_s, set_marker_off, (size_t)(nsets + 1))) ||
+      (rc = mem.upload(&d_c, marker_count, (size_t)nm)) || (rc = mem.get(&d_o, (size_t)nbins))) return rc;
+  genome_check_kernel<<<(nbins + 127) / 128, 128, 0, st>>>(nbins, d_b, d_s, d_c, individual_markers, d_o);
+  CKM_CUDA(cudaGetLastError());
+  CKM_CUDA(cudaMemcpyAsync(rows_out, d_o, sizeof(ckm_qa_row) * nbins, cudaMemcpyDeviceToHost, st));
+  CKM_CUDA(cudaStreamSynchronize(st));
   e->stats.kernel_launches++;
   return CKM_OK;
 }
@@ -396,41 +413,33 @@ static int reduce_once(ckm_engine *e, int32_t nmodels_in, int32_t nseq_in, int32
   const int64_t nsetm = (meta->set_marker_off && nsets > 0) ? meta->set_marker_off[nsets] : 0;
   std::vector<int64_t> zero_off(nbins + 1, 0), zero_set(1, 0);
 
-  std::vector<void *> frees;
-  auto dalloc = [&](size_t bytes) -> void * { void *p = nullptr; if (cudaMallocAsync(&p, std::max<size_t>(bytes, 16), st) != cudaSuccess) return nullptr; frees.push_back(p); return p; };
-  auto cleanup = [&]() { for (void *p : frees) cudaFreeAsync(p, st); };
-#define RCUDA(call) do { cudaError_t _e = (call); if (_e != cudaSuccess) { cleanup(); return cuda_fail(_e, #call); } } while (0)
-#define UP(dst, src, bytes) do { dst = (decltype(dst))dalloc(bytes); if (!dst) { cleanup(); set_error("ckm_reduce: out of device memory"); return CKM_ENOMEM; } if ((bytes) > 0) RCUDA(cudaMemcpyAsync((void *)dst, src, bytes, cudaMemcpyHostToDevice, st)); } while (0)
   RParams p;
   std::memset(&p, 0, sizeof(p));
   p.nhits = nhits; p.nseg = nseg; p.nbins = nbins; p.nmodels = nmodels; p.opts = *opts;
-  const size_t nh = (size_t)std::max<int64_t>(nhits, 1);
-  ckm_hit *d_hits; UP(d_hits, hits, sizeof(ckm_hit) * (size_t)nhits); p.hits = d_hits;
-  if (meta->row_scores != nullptr && nhits > 0) { double *d_rs; UP(d_rs, meta->row_scores, sizeof(double) * 2 * (size_t)nhits); p.row_scores = d_rs; }
-  p.rows = (RRow *)dalloc(sizeof(RRow) * nh); p.list = (int32_t *)dalloc(sizeof(int32_t) * nh); p.list_len = (int32_t *)dalloc(sizeof(int32_t) * std::max(nseg, 1));
-  p.filtered = (uint8_t *)dalloc(nh); p.first_app = (int64_t *)dalloc(sizeof(int64_t) * nh);
-  p.mh = (ckm_marker_hit *)dalloc(sizeof(ckm_marker_hit) * nh); p.mh_len = (int32_t *)dalloc(sizeof(int32_t) * std::max(nseg, 1));
-  p.qa = (ckm_qa_row *)dalloc(sizeof(ckm_qa_row) * nbins);
-  int32_t *d_overflow = (int32_t *)dalloc(sizeof(int32_t));
-  if (!p.rows || !p.list || !p.list_len || !p.filtered || !p.first_app || !p.mh || !p.mh_len || !p.qa || !d_overflow) { cleanup(); set_error("ckm_reduce: out of device memory"); return CKM_ENOMEM; }
-  RCUDA(cudaMemsetAsync(d_overflow, 0, sizeof(int32_t), st));
-  RCUDA(cudaMemsetAsync(p.mh_len, 0, sizeof(int32_t) * std::max(nseg, 1), st));
-  RModel *d_rm; UP(d_rm, rm.data(), sizeof(RModel) * rm.size()); p.models = d_rm;
-  int64_t *d_no; UP(d_no, nest_off, sizeof(int64_t) * (nmodels + 1)); p.nest_off = d_no;
-  int32_t *d_ni; UP(d_ni, meta->nest_idx, sizeof(int32_t) * (size_t)nnest); p.nest_idx = d_ni;
+  const size_t nh = (size_t)std::max<int64_t>(nhits, 1), ns = (size_t)std::max(nseg, 1);
+  CallBuffers mem(st, "ckm_reduce");
+  int32_t *d_overflow;
+  int rc;
+  if ((rc = mem.upload(&p.hits, hits, (size_t)nhits))) return rc;
+  if (meta->row_scores != nullptr && nhits > 0 && (rc = mem.upload(&p.row_scores, meta->row_scores, 2 * (size_t)nhits))) return rc;
+  if ((rc = mem.get(&p.rows, nh)) || (rc = mem.get(&p.list, nh)) || (rc = mem.get(&p.list_len, ns)) || (rc = mem.get(&p.filtered, nh)) ||
+      (rc = mem.get(&p.first_app, nh)) || (rc = mem.get(&p.mh, nh)) || (rc = mem.get(&p.mh_len, ns)) || (rc = mem.get(&p.qa, (size_t)nbins)) ||
+      (rc = mem.get(&d_overflow, 1))) return rc;
+  CKM_CUDA(cudaMemsetAsync(d_overflow, 0, sizeof(int32_t), st));
+  CKM_CUDA(cudaMemsetAsync(p.mh_len, 0, sizeof(int32_t) * ns, st));
   std::vector<int32_t> zero_seq(std::max(nseq, 1), 0);
-  int32_t *d_sc; UP(d_sc, meta->scaffold_id ? meta->scaffold_id : zero_seq.data(), sizeof(int32_t) * (size_t)nseq); p.scaffold_id = d_sc;
-  int32_t *d_on; UP(d_on, meta->orf_num ? meta->orf_num : zero_seq.data(), sizeof(int32_t) * (size_t)nseq); p.orf_num = d_on;
-  int32_t *d_nr; UP(d_nr, meta->name_rank ? meta->name_rank : zero_seq.data(), sizeof(int32_t) * (size_t)nseq); p.name_rank = d_nr;
-  int64_t *d_so; UP(d_so, seg_off.data(), sizeof(int64_t) * seg_off.size()); p.seg_off = d_so;
-  int32_t *d_sb; UP(d_sb, seg_bin.data(), sizeof(int32_t) * seg_bin.size()); p.seg_bin = d_sb;
-  int32_t *d_sm; UP(d_sm, seg_model.data(), sizeof(int32_t) * seg_model.size()); p.seg_model = d_sm;
-  int64_t *d_bro; UP(d_bro, bin_row_off.data(), sizeof(int64_t) * bin_row_off.size()); p.bin_row_off = d_bro;
-  int64_t *d_bso; UP(d_bso, bin_seg_off.data(), sizeof(int64_t) * bin_seg_off.size()); p.bin_seg_off = d_bso;
-  int64_t *d_bs; UP(d_bs, meta->bin_set_off ? meta->bin_set_off : zero_off.data(), sizeof(int64_t) * (nbins + 1)); p.bin_set_off = d_bs;
-  int64_t *d_smo; UP(d_smo, (meta->set_marker_off && nsets > 0) ? meta->set_marker_off : zero_set.data(), sizeof(int64_t) * (size_t)(nsets + 1)); p.set_marker_off = d_smo;
-  int32_t *d_smi; UP(d_smi, meta->set_marker_idx, sizeof(int32_t) * (size_t)nsetm); p.set_marker_idx = d_smi;
-  int32_t *d_sof; UP(d_sof, seg_of.data(), sizeof(int32_t) * seg_of.size()); p.seg_of_bin_model = d_sof;
+  if ((rc = mem.upload(&p.models, rm.data(), rm.size())) || (rc = mem.upload(&p.nest_off, nest_off, (size_t)nmodels + 1)) ||
+      (rc = mem.upload(&p.nest_idx, meta->nest_idx, (size_t)nnest)) ||
+      (rc = mem.upload(&p.scaffold_id, meta->scaffold_id ? meta->scaffold_id : zero_seq.data(), (size_t)nseq)) ||
+      (rc = mem.upload(&p.orf_num, meta->orf_num ? meta->orf_num : zero_seq.data(), (size_t)nseq)) ||
+      (rc = mem.upload(&p.name_rank, meta->name_rank ? meta->name_rank : zero_seq.data(), (size_t)nseq)) ||
+      (rc = mem.upload(&p.seg_off, seg_off.data(), seg_off.size())) || (rc = mem.upload(&p.seg_bin, seg_bin.data(), seg_bin.size())) ||
+      (rc = mem.upload(&p.seg_model, seg_model.data(), seg_model.size())) || (rc = mem.upload(&p.bin_row_off, bin_row_off.data(), bin_row_off.size())) ||
+      (rc = mem.upload(&p.bin_seg_off, bin_seg_off.data(), bin_seg_off.size())) ||
+      (rc = mem.upload(&p.bin_set_off, meta->bin_set_off ? meta->bin_set_off : zero_off.data(), (size_t)nbins + 1)) ||
+      (rc = mem.upload(&p.set_marker_off, (meta->set_marker_off && nsets > 0) ? meta->set_marker_off : zero_set.data(), (size_t)(nsets + 1))) ||
+      (rc = mem.upload(&p.set_marker_idx, meta->set_marker_idx, (size_t)nsetm)) ||
+      (rc = mem.upload(&p.seg_of_bin_model, seg_of.data(), seg_of.size()))) return rc;
 
   const int T = 128;
   if (nhits > 0) {
@@ -440,20 +449,19 @@ static int reduce_once(ckm_engine *e, int32_t nmodels_in, int32_t nseq_in, int32
     r3_adjacent<<<(nseg + T - 1) / T, T, 0, st>>>(p);
   }
   r4_counts<<<(nbins + T - 1) / T, T, 0, st>>>(p);
-  RCUDA(cudaGetLastError());
+  CKM_CUDA(cudaGetLastError());
   e->stats.kernel_launches += 5;
   std::vector<ckm_marker_hit> mh((size_t)nhits);
   std::vector<int32_t> mh_len(std::max(nseg, 1), 0);
   ckm_qa_row *qa = (ckm_qa_row *)std::malloc(sizeof(ckm_qa_row) * std::max(nbins, 1));
   int32_t overflow = 0;
   if (nhits > 0) {
-    RCUDA(cudaMemcpyAsync(mh.data(), p.mh, sizeof(ckm_marker_hit) * (size_t)nhits, cudaMemcpyDeviceToHost, st));
-    RCUDA(cudaMemcpyAsync(mh_len.data(), p.mh_len, sizeof(int32_t) * nseg, cudaMemcpyDeviceToHost, st));
+    CKM_CUDA(cudaMemcpyAsync(mh.data(), p.mh, sizeof(ckm_marker_hit) * (size_t)nhits, cudaMemcpyDeviceToHost, st));
+    CKM_CUDA(cudaMemcpyAsync(mh_len.data(), p.mh_len, sizeof(int32_t) * nseg, cudaMemcpyDeviceToHost, st));
   }
-  RCUDA(cudaMemcpyAsync(qa, p.qa, sizeof(ckm_qa_row) * nbins, cudaMemcpyDeviceToHost, st));
-  RCUDA(cudaMemcpyAsync(&overflow, d_overflow, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  RCUDA(cudaStreamSynchronize(st));
-  cleanup();
+  CKM_CUDA(cudaMemcpyAsync(qa, p.qa, sizeof(ckm_qa_row) * nbins, cudaMemcpyDeviceToHost, st));
+  CKM_CUDA(cudaMemcpyAsync(&overflow, d_overflow, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CKM_CUDA(cudaStreamSynchronize(st));
   if (overflow) { std::free(qa); set_error("ckm_reduce: more than 384 Pfam hits on one ORF"); return CKM_ECAPACITY; }
   // compact the per-segment lists
   int64_t total = 0;
@@ -466,13 +474,13 @@ static int reduce_once(ckm_engine *e, int32_t nmodels_in, int32_t nseq_in, int32
   return CKM_OK;
 }
 
-// Frees what the engine keeps cached between calls: its search workspaces (the next search allocates them again) and the
-// unused blocks of the device's stream-ordered pool.
+// Frees what the engine keeps cached between calls: its workspaces (the next call allocates them again) and the unused blocks
+// of the device's stream-ordered pool.
 static void release_cached_memory(ckm_engine *e) {
   cudaStreamSynchronize(e->stream);
   for (auto &s : e->cls) cudaStreamSynchronize(s);
   if (e->aux) cudaStreamSynchronize(e->aux);
-  for (auto &ent : e->pool) { cudaFree(ent.first); ent = std::make_pair((void *)nullptr, (size_t)0); }
+  workspace_release(e);
   cudaMemPool_t mp;
   if (cudaDeviceGetDefaultMemPool(&mp, e->device) == cudaSuccess) cudaMemPoolTrimTo(mp, 0);
 }
@@ -482,7 +490,7 @@ extern "C" int ckm_reduce(ckm_engine *e, int32_t nmodels_in, int32_t nseq_in, in
                           ckm_qa_row **qa_out, int32_t *nqa_out, ckm_marker_hit **mh_out, int64_t *nmh_out) {
   int rc = reduce_once(e, nmodels_in, nseq_in, nbins_in, hits, nhits, opts, meta, qa_out, nqa_out, mh_out, nmh_out);
   if (rc == CKM_ENOMEM) {
-    // after a large search the engine's cached workspaces can hold most of the device: a reduction over many bins
+    // after a large search the engine's workspaces can hold most of the device: a reduction over many bins
     // (one analyseResults over a whole directory) then finds no room for its rows
     cudaGetLastError();              // the failed allocation must not surface as a launch error of the retry
     release_cached_memory(e);

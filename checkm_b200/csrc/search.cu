@@ -17,8 +17,6 @@ using namespace ckm;
 namespace ckm {
 
 std::atomic<int> g_live_engines{0};     // engines alive in this process: they share the envelope-scratch budget
-thread_local ckm_engine *g_pool_engine = nullptr;
-thread_local int g_pool_next = 0;
 
 static bool use_blocked_kernels();
 static bool use_packed_viterbi() { const char *v = std::getenv("CKM_VITP"); return use_blocked_kernels() && !(v != nullptr && v[0] == '0'); }
@@ -27,13 +25,14 @@ static int fan_in(ckm_engine *e);
 enum { CTR_UNIT4 = 0, CTR_UNIT8, CTR_UNIT16, CTR_UNIT32, CTR_CAND, CTR_MSV, CTR_BIAS, CTR_VIT, CTR_FWD, CTR_ENV, CTR_DOM, CTR_VREDO, CTR_SSVRES, CTR_VWORK = 16 /* .. 25: cursors of the packed-Viterbi class kernels */, CTR_N = 32 };
 
 struct ActiveMasks {
-  DevBuf tile_active, model_active, model_slot;
-  bool all_active = true;
+  int32_t *model_slot = nullptr;
+  uint8_t *tile_active = nullptr, *model_active = nullptr;    // nullptr: every model is queried in every bin
 };
 
 // Builds the per-bin activity masks for a query subset.  bin_model_offsets == nullptr: the same nmodels queries for all bins.
-static int build_masks(const ckm_models *m, const ckm_seqdb *db, const int32_t *model_idx, int32_t nmodels,
-                       const int64_t *bin_model_offsets, ActiveMasks &am, std::vector<int32_t> &slot_of_model, cudaStream_t st) {
+static int build_masks(ckm_engine *e, const ckm_models *m, const ckm_seqdb *db, const int32_t *model_idx, int32_t nmodels,
+                       const int64_t *bin_model_offsets, ActiveMasks &am, std::vector<int32_t> &slot_of_model) {
+  cudaStream_t st = e->stream;
   const int ndb = (int)m->models.size(), nbins = db->nbins, ntiles = (int)m->tiles.size();
   slot_of_model.assign(ndb, -1);
   bool all = (bin_model_offsets == nullptr) && (model_idx == nullptr || nmodels == ndb);
@@ -46,10 +45,9 @@ static int build_masks(const ckm_models *m, const ckm_seqdb *db, const int32_t *
     }
     if (all) for (int i = 0; i < ndb; ++i) if (slot_of_model[i] < 0) all = false;
   }
-  am.all_active = all;
   int rc;
-  if ((rc = am.model_slot.alloc(sizeof(int32_t) * ndb))) return rc;
-  CKM_CUDA(cudaMemcpyAsync(am.model_slot.p, slot_of_model.data(), sizeof(int32_t) * ndb, cudaMemcpyHostToDevice, st));
+  if ((rc = workspace(e, Ws::ModelSlot, sizeof(int32_t) * ndb, &am.model_slot))) return rc;
+  CKM_CUDA(cudaMemcpyAsync(am.model_slot, slot_of_model.data(), sizeof(int32_t) * ndb, cudaMemcpyHostToDevice, st));
   if (all) return CKM_OK;
   std::vector<uint8_t> ma((size_t)nbins * ndb, 0), ta((size_t)nbins * ntiles, 0);
   for (int b = 0; b < nbins; ++b) {
@@ -69,17 +67,17 @@ static int build_masks(const ckm_models *m, const ckm_seqdb *db, const int32_t *
     }
     // a chained model is addressed through its first tile
   }
-  if ((rc = am.model_active.alloc(ma.size()))) return rc;
-  if ((rc = am.tile_active.alloc(ta.size()))) return rc;
-  CKM_CUDA(cudaMemcpyAsync(am.model_active.p, ma.data(), ma.size(), cudaMemcpyHostToDevice, st));
-  CKM_CUDA(cudaMemcpyAsync(am.tile_active.p, ta.data(), ta.size(), cudaMemcpyHostToDevice, st));
+  if ((rc = workspace(e, Ws::ModelActive, ma.size(), &am.model_active))) return rc;
+  if ((rc = workspace(e, Ws::TileActive, ta.size(), &am.tile_active))) return rc;
+  CKM_CUDA(cudaMemcpyAsync(am.model_active, ma.data(), ma.size(), cudaMemcpyHostToDevice, st));
+  CKM_CUDA(cudaMemcpyAsync(am.tile_active, ta.data(), ta.size(), cudaMemcpyHostToDevice, st));
   CKM_CUDA(cudaStreamSynchronize(st));     // host vectors go out of scope
   return CKM_OK;
 }
 
 // Stage 1: SSV pre-filter over all pairs -> candidate list; exact MSV on the candidates -> pass list.
 struct Stage1 {
-  DevBuf cand, pass, bnd, glist, cells;
+  int2 *cand = nullptr; Candidate *pass = nullptr; unsigned long long *cells = nullptr;
   int32_t cand_cap = 0, pass_cap = 0;
 };
 
@@ -101,24 +99,26 @@ static int run_stage1(ckm_engine *e, const ckm_models *m, const ckm_seqdb *db, A
   const int64_t n_bypass = (int64_t)m->ssv_bypass.size() * db->nseq;          // models without SSV tiles: every pair is a candidate
   s1.cand_cap = (int32_t)std::min<int64_t>(QUEUE_MAX, (int64_t)s1.cand_cap + n_bypass);
   s1.pass_cap = queue_cap(n_pairs, 12, attempt);
-  if ((rc = s1.cand.alloc(sizeof(int2) * (size_t)s1.cand_cap))) return rc;
-  if ((rc = s1.pass.alloc(sizeof(Candidate) * (size_t)s1.pass_cap))) return rc;
-  if ((rc = s1.cells.alloc(sizeof(unsigned long long)))) return rc;
+  if ((rc = workspace(e, Ws::Cand, sizeof(int2) * (size_t)s1.cand_cap, &s1.cand))) return rc;
+  if ((rc = workspace(e, Ws::Pass, sizeof(Candidate) * (size_t)s1.pass_cap, &s1.pass))) return rc;
+  if ((rc = workspace(e, Ws::Cells, sizeof(unsigned long long), &s1.cells))) return rc;
   CKM_CUDA(cudaMemsetAsync(e->d_counters, 0, CTR_N * sizeof(int32_t), st));
-  CKM_CUDA(cudaMemsetAsync(s1.cells.p, 0, sizeof(unsigned long long), st));
+  CKM_CUDA(cudaMemsetAsync(s1.cells, 0, sizeof(unsigned long long), st));
   const int nsm = e->prop.multiProcessorCount;
   bool need_bnd = false;
   for (int nt : m->chain_ntiles) need_bnd |= (nt > 1);
   const int64_t bnd_stride = ((int64_t)db->maxL + 31) / 16 * 16;
-  if (need_bnd) { if ((rc = s1.bnd.alloc((size_t)nsm * SSV_WARPS_HOST * 2 * bnd_stride * sizeof(int16_t)))) return rc; }
+  int16_t *bnd = nullptr;
+  if (need_bnd) { if ((rc = workspace(e, Ws::Bnd, (size_t)nsm * SSV_WARPS_HOST * 2 * bnd_stride * sizeof(int16_t), &bnd))) return rc; }
   // group lists per J
   std::vector<int32_t> gl[4];
   for (size_t g = 0; g < m->groups.size(); ++g) gl[m->groups[g].J == 4 ? 0 : (m->groups[g].J == 8 ? 1 : (m->groups[g].J == 16 ? 2 : 3))].push_back((int32_t)g);
   std::vector<int32_t> flat;
   size_t goff[4];
   for (int c = 0; c < 4; ++c) { goff[c] = flat.size(); flat.insert(flat.end(), gl[c].begin(), gl[c].end()); }
-  if ((rc = s1.glist.alloc(sizeof(int32_t) * std::max<size_t>(flat.size(), 1)))) return rc;
-  if (!flat.empty()) CKM_CUDA(cudaMemcpyAsync(s1.glist.p, flat.data(), sizeof(int32_t) * flat.size(), cudaMemcpyHostToDevice, st));
+  int32_t *glist;
+  if ((rc = workspace(e, Ws::GroupList, sizeof(int32_t) * std::max<size_t>(flat.size(), 1), &glist))) return rc;
+  if (!flat.empty()) CKM_CUDA(cudaMemcpyAsync(glist, flat.data(), sizeof(int32_t) * flat.size(), cudaMemcpyHostToDevice, st));
   CKM_CUDA(cudaStreamSynchronize(st));
 
   CKM_CUDA(cudaEventRecord(e->ev[0], st));
@@ -131,22 +131,21 @@ static int run_stage1(ckm_engine *e, const ckm_models *m, const ckm_seqdb *db, A
     p.nseq = db->nseq;
     p.seq_chunk = 128;
     p.nchunks = (db->nseq + p.seq_chunk - 1) / p.seq_chunk;
-    p.groups = m->d_groups; p.group_list = s1.glist.as<int32_t>() + goff[c]; p.ngroups = (int32_t)gl[c].size();
+    p.groups = m->d_groups; p.group_list = glist + goff[c]; p.ngroups = (int32_t)gl[c].size();
     p.tiles = m->d_tiles; p.tile_models = m->d_tile_models;
     p.chain_first_tile = m->d_chain_first_tile; p.chain_ntiles = m->d_chain_ntiles;
     p.tile_blob = m->d_tile_blob;
-    p.tile_active = am.all_active ? nullptr : am.tile_active.as<uint8_t>();
-    p.model_active = am.all_active ? nullptr : am.model_active.as<uint8_t>();
+    p.tile_active = am.tile_active; p.model_active = am.model_active;
     p.ntiles = (int32_t)m->tiles.size(); p.nmodels = (int32_t)m->models.size();
     p.unit_counter = e->d_counters + CTR_UNIT4 + c;
-    p.cand = s1.cand.as<int2>(); p.cand_count = e->d_counters + CTR_CAND; p.cand_cap = s1.cand_cap;
-    p.bnd = need_bnd ? s1.bnd.as<int16_t>() : nullptr; p.bnd_stride = bnd_stride;
-    p.cells = s1.cells.as<unsigned long long>();
+    p.cand = s1.cand; p.cand_count = e->d_counters + CTR_CAND; p.cand_cap = s1.cand_cap;
+    p.bnd = bnd; p.bnd_stride = bnd_stride;
+    p.cells = s1.cells;
     { const char *v = std::getenv("CKM_SSV_RESOLVE"); p.resolve = (v != nullptr && v[0] == '0') ? 0 : 1; }
     p.ms = m->d_scalars; p.nullsc = db->d_nullsc;
-    p.pass = s1.pass.as<Candidate>(); p.pass_count = e->d_counters + CTR_MSV; p.pass_cap = s1.pass_cap;
+    p.pass = s1.pass; p.pass_count = e->d_counters + CTR_MSV; p.pass_cap = s1.pass_cap;
     p.resolved_count = e->d_counters + CTR_SSVRES;
-    p.xj_dense = xj_dense; p.model_slot = am.model_slot.as<int32_t>();
+    p.xj_dense = xj_dense; p.model_slot = am.model_slot;
     p.F1 = 0.02;
     int64_t maxbytes = 0;
     for (int g : gl[c]) maxbytes = std::max<int64_t>(maxbytes, m->groups[g].table_bytes);
@@ -157,8 +156,7 @@ static int run_stage1(ckm_engine *e, const ckm_models *m, const ckm_seqdb *db, A
   }
   if (!m->ssv_bypass.empty()) {
     if ((rc = launch_ssv_bypass(m->d_ssv_bypass, (int32_t)m->ssv_bypass.size(), db->nseq, db->d_len, db->d_bin,
-                                am.all_active ? nullptr : am.model_active.as<uint8_t>(), (int32_t)m->models.size(),
-                                s1.cand.as<int2>(), e->d_counters + CTR_CAND, s1.cand_cap, st))) return rc;
+                                am.model_active, (int32_t)m->models.size(), s1.cand, e->d_counters + CTR_CAND, s1.cand_cap, st))) return rc;
     e->stats.kernel_launches++;
   }
   CKM_CUDA(cudaEventRecord(e->ev[1], st));
@@ -167,9 +165,9 @@ static int run_stage1(ckm_engine *e, const ckm_models *m, const ckm_seqdb *db, A
     MsvParams p{};
     p.res = db->d_res; p.off = db->d_off; p.len = db->d_len; p.nullsc = db->d_nullsc; p.tjb = db->d_tjb;
     p.ms = m->d_scalars; p.rbv = m->d_rbv; p.rmb = m->d_rmb;
-    p.cand = s1.cand.as<int2>(); p.cand_count = e->d_counters + CTR_CAND; p.cand_cap = s1.cand_cap;
-    p.out = s1.pass.as<Candidate>(); p.out_count = e->d_counters + CTR_MSV; p.out_cap = s1.pass_cap;
-    p.xj_dense = xj_dense; p.model_slot = am.model_slot.as<int32_t>(); p.nseq = db->nseq;
+    p.cand = s1.cand; p.cand_count = e->d_counters + CTR_CAND; p.cand_cap = s1.cand_cap;
+    p.out = s1.pass; p.out_count = e->d_counters + CTR_MSV; p.out_cap = s1.pass_cap;
+    p.xj_dense = xj_dense; p.model_slot = am.model_slot; p.nseq = db->nseq;
     p.row_bytes = (m->maxM + 2 + 15) / 16 * 16;
     p.F1 = 0.02;
     p.use_blk = use_blocked_kernels() ? 1 : 0;
@@ -186,7 +184,7 @@ static int run_stage1(ckm_engine *e, const ckm_models *m, const ckm_seqdb *db, A
 
 // Stages 2-4 on the MSV survivors: bias filter -> ViterbiFilter -> ForwardParser.  Lists ping-pong between two buffers.
 struct Stage2 {
-  DevBuf a, b, redo;
+  Candidate *a = nullptr, *b = nullptr, *redo = nullptr;
   int32_t cap = 0;
   Candidate *fwd_list = nullptr;      // survivors of the Forward filter (points into a or b)
 };
@@ -196,29 +194,29 @@ static int run_stage2(ckm_engine *e, const ckm_models *m, const ckm_seqdb *db, A
   cudaStream_t st = e->stream;
   int rc;
   s2.cap = s1.pass_cap;
-  if ((rc = s2.a.alloc(sizeof(Candidate) * (size_t)s2.cap))) return rc;
-  if ((rc = s2.b.alloc(sizeof(Candidate) * (size_t)s2.cap))) return rc;
-  if ((rc = s2.redo.alloc(sizeof(Candidate) * (size_t)s2.cap))) return rc;
+  if ((rc = workspace(e, Ws::ListA, sizeof(Candidate) * (size_t)s2.cap, &s2.a))) return rc;
+  if ((rc = workspace(e, Ws::ListB, sizeof(Candidate) * (size_t)s2.cap, &s2.b))) return rc;
+  if ((rc = workspace(e, Ws::Redo, sizeof(Candidate) * (size_t)s2.cap, &s2.redo))) return rc;
   const int nsm = e->prop.multiProcessorCount;
   FilterParams p{};
   p.res = db->d_res; p.off = db->d_off; p.len = db->d_len; p.lenA = db->d_lenA; p.lenB = db->d_lenB; p.tmove_w = db->d_tmove_w;
   p.ms = m->d_scalars; p.bias_eo = m->d_bias_eo; p.rwv = m->d_rwv; p.twv = m->d_twv; p.rfv = m->d_rfv; p.tfv = m->d_tfv;
   p.twb = m->d_twb; p.rwb = m->d_rwb; p.tfb = m->d_tfb; p.rfb = m->d_rfb;
   p.twp = m->d_twp; p.rwp = m->d_rwp;
-  p.redo = s2.redo.as<Candidate>(); p.redo_count = e->d_counters + CTR_VREDO; p.redo_cap = s2.cap;
+  p.redo = s2.redo; p.redo_count = e->d_counters + CTR_VREDO; p.redo_cap = s2.cap;
   p.row_elems = ((m->maxM + 31) / 32) * 32 + 64;
   p.F1 = 0.02; p.F2 = 1e-3; p.F3 = 1e-5;
   p.use_blk = use_blocked_kernels() ? 1 : 0;
   p.dense_filtersc = d_filtersc; p.dense_vit = d_vit; p.dense_fwd = d_fwd; p.dense_passed = d_passed;
-  p.model_slot = am.model_slot.as<int32_t>(); p.nseq = db->nseq;
+  p.model_slot = am.model_slot; p.nseq = db->nseq;
   // bias: pass list (stage 1) -> a
-  p.in = s1.pass.as<Candidate>(); p.in_count = e->d_counters + CTR_MSV; p.in_cap = s1.pass_cap;
-  p.out = s2.a.as<Candidate>(); p.out_count = e->d_counters + CTR_BIAS; p.out_cap = s2.cap;
+  p.in = s1.pass; p.in_count = e->d_counters + CTR_MSV; p.in_cap = s1.pass_cap;
+  p.out = s2.a; p.out_count = e->d_counters + CTR_BIAS; p.out_cap = s2.cap;
   if ((rc = launch_bias(p, nsm * 8, st))) return rc;
   CKM_CUDA(cudaEventRecord(e->ev[3], st));
   // viterbi: a -> b
-  p.in = s2.a.as<Candidate>(); p.in_count = e->d_counters + CTR_BIAS; p.in_cap = s2.cap;
-  p.out = s2.b.as<Candidate>(); p.out_count = e->d_counters + CTR_VIT; p.out_cap = s2.cap;
+  p.in = s2.a; p.in_count = e->d_counters + CTR_BIAS; p.in_cap = s2.cap;
+  p.out = s2.b; p.out_count = e->d_counters + CTR_VIT; p.out_cap = s2.cap;
   if (use_packed_viterbi()) {
     // packed int16x2 kernels, one per class; what they cannot score exactly (strong hits near the int16 ceiling, models
     // without a class, pairs outside the safety conditions of kernels_vitp.cu) lands in the redo list ...
@@ -227,7 +225,7 @@ static int run_stage2(ckm_engine *e, const ckm_models *m, const ckm_seqdb *db, A
     for (int c = 0; c < N_BLK_CLASSES; ++c) if ((rc = launch_vitp(p, c, nsm * 8, e->cls[c]))) return rc;
     if ((rc = fan_in(e))) return rc;
     // ... which the int32 kernels below then take as their input
-    p.in = s2.redo.as<Candidate>(); p.in_count = e->d_counters + CTR_VREDO; p.in_cap = s2.cap;
+    p.in = s2.redo; p.in_count = e->d_counters + CTR_VREDO; p.in_cap = s2.cap;
     e->stats.kernel_launches += N_BLK_CLASSES;
   }
   if ((rc = fan_out(e))) return rc;
@@ -236,8 +234,8 @@ static int run_stage2(ckm_engine *e, const ckm_models *m, const ckm_seqdb *db, A
   if ((rc = fan_in(e))) return rc;
   CKM_CUDA(cudaEventRecord(e->ev[4], st));
   // forward: b -> a
-  p.in = s2.b.as<Candidate>(); p.in_count = e->d_counters + CTR_VIT; p.in_cap = s2.cap;
-  p.out = s2.a.as<Candidate>(); p.out_count = e->d_counters + CTR_FWD; p.out_cap = s2.cap;
+  p.in = s2.b; p.in_count = e->d_counters + CTR_VIT; p.in_cap = s2.cap;
+  p.out = s2.a; p.out_count = e->d_counters + CTR_FWD; p.out_cap = s2.cap;
   if ((rc = fan_out(e))) return rc;
   // widest classes first: their one-warp-per-pair kernels are the long pole of the stage, the narrow ones fill in around them
   if ((rc = launch_fwd(p, nsm * 4, e->cls[N_BLK_CLASSES]))) return rc;
@@ -245,7 +243,7 @@ static int run_stage2(ckm_engine *e, const ckm_models *m, const ckm_seqdb *db, A
   if ((rc = fan_in(e))) return rc;
   CKM_CUDA(cudaEventRecord(e->ev[5], st));
   e->stats.kernel_launches += 3 + (p.use_blk ? 2 * N_BLK_CLASSES : 0);
-  s2.fwd_list = s2.a.as<Candidate>();
+  s2.fwd_list = s2.a;
   return CKM_OK;
 }
 
@@ -258,36 +256,35 @@ int ckm_filter_scores(ckm_engine *e, const ckm_models *m, const int32_t *model_i
   if (!e || !m || !db || !filtersc_out || !vit_out || !fwd_out || !passed_out) { set_error("ckm_filter_scores: bad argument"); return CKM_EINVAL; }
   cudaSetDevice(e->device);
   if (model_idx == nullptr) nmodels = (int32_t)m->models.size();
-  PoolScope pool_scope(e);
   ActiveMasks am; std::vector<int32_t> slot;
-  int rc = build_masks(m, db, model_idx, nmodels, nullptr, am, slot, e->stream);
+  int rc = build_masks(e, m, db, model_idx, nmodels, nullptr, am, slot);
   if (rc) return rc;
   const int64_t n = (int64_t)nmodels * db->nseq;
-  DevBuf dfs, dvit, dfwd, dpass;
+  float *dfs, *dvit, *dfwd; uint8_t *dpass;
   const size_t nf = (size_t)std::max<int64_t>(n, 1);
-  if ((rc = dfs.alloc(sizeof(float) * nf)) || (rc = dvit.alloc(sizeof(float) * nf)) || (rc = dfwd.alloc(sizeof(float) * nf)) ||
-      (rc = dpass.alloc(nf + 4))) return rc;
+  if ((rc = workspace(e, Ws::DenseFiltersc, sizeof(float) * nf, &dfs)) || (rc = workspace(e, Ws::DenseVit, sizeof(float) * nf, &dvit)) ||
+      (rc = workspace(e, Ws::DenseFwd, sizeof(float) * nf, &dfwd)) || (rc = workspace(e, Ws::DensePassed, nf + 4, &dpass))) return rc;
   // NaN-fill the float outputs, zero the flags
-  CKM_CUDA(cudaMemsetAsync(dfs.p, 0xff, sizeof(float) * nf, e->stream));
-  CKM_CUDA(cudaMemsetAsync(dvit.p, 0xff, sizeof(float) * nf, e->stream));
-  CKM_CUDA(cudaMemsetAsync(dfwd.p, 0xff, sizeof(float) * nf, e->stream));
-  CKM_CUDA(cudaMemsetAsync(dpass.p, 0, nf + 4, e->stream));
+  CKM_CUDA(cudaMemsetAsync(dfs, 0xff, sizeof(float) * nf, e->stream));
+  CKM_CUDA(cudaMemsetAsync(dvit, 0xff, sizeof(float) * nf, e->stream));
+  CKM_CUDA(cudaMemsetAsync(dfwd, 0xff, sizeof(float) * nf, e->stream));
+  CKM_CUDA(cudaMemsetAsync(dpass, 0, nf + 4, e->stream));
   Stage1 s1; Stage2 s2;
   std::memset(&e->stats, 0, sizeof(e->stats));
   if ((rc = run_stage1(e, m, db, am, n, s1, nullptr))) return rc;
-  if ((rc = run_stage2(e, m, db, am, s1, s2, dfs.as<float>(), dvit.as<float>(), dfwd.as<float>(), dpass.as<uint8_t>()))) return rc;
+  if ((rc = run_stage2(e, m, db, am, s1, s2, dfs, dvit, dfwd, dpass))) return rc;
   int32_t ctr[CTR_N];
   CKM_CUDA(cudaMemcpyAsync(ctr, e->d_counters, sizeof(ctr), cudaMemcpyDeviceToHost, e->stream));
-  CKM_CUDA(cudaMemcpyAsync(filtersc_out, dfs.p, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
-  CKM_CUDA(cudaMemcpyAsync(vit_out, dvit.p, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
-  CKM_CUDA(cudaMemcpyAsync(fwd_out, dfwd.p, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
-  CKM_CUDA(cudaMemcpyAsync(passed_out, dpass.p, (size_t)n, cudaMemcpyDeviceToHost, e->stream));
+  CKM_CUDA(cudaMemcpyAsync(filtersc_out, dfs, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
+  CKM_CUDA(cudaMemcpyAsync(vit_out, dvit, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
+  CKM_CUDA(cudaMemcpyAsync(fwd_out, dfwd, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
+  CKM_CUDA(cudaMemcpyAsync(passed_out, dpass, (size_t)n, cudaMemcpyDeviceToHost, e->stream));
   std::vector<Candidate> pass1((size_t)std::min<int64_t>(s1.pass_cap, std::max<int32_t>(1, s1.pass_cap)));
   CKM_CUDA(cudaStreamSynchronize(e->stream));
   if (ctr[CTR_CAND] > s1.cand_cap || ctr[CTR_MSV] > s1.pass_cap) { set_error("candidate queue overflow"); return CKM_ECAPACITY; }
   // MSV pass flags come from the stage-1 pass list
   pass1.resize((size_t)ctr[CTR_MSV]);
-  if (!pass1.empty()) CKM_CUDA(cudaMemcpy(pass1.data(), s1.pass.p, sizeof(Candidate) * pass1.size(), cudaMemcpyDeviceToHost));
+  if (!pass1.empty()) CKM_CUDA(cudaMemcpy(pass1.data(), s1.pass, sizeof(Candidate) * pass1.size(), cudaMemcpyDeviceToHost));
   for (const Candidate &c : pass1) passed_out[(int64_t)slot[c.model] * db->nseq + c.seq] |= 1;
   e->stats.n_pairs = n;
   e->stats.n_ssv_cand = (int64_t)ctr[CTR_CAND] + ctr[CTR_SSVRES]; e->stats.n_msv_exact = ctr[CTR_CAND]; e->stats.n_past_msv = ctr[CTR_MSV]; e->stats.n_past_bias = ctr[CTR_BIAS];
@@ -348,13 +345,12 @@ static std::vector<float> &logsum_table() {
 // Envelope rescoring in waves: one matrix (blocked kernels; two for the chunked ones) + specials of scratch per envelope under a fixed budget, every class on its own
 // stream.  leave_last: the last wave is left running on the class streams (the caller joins them with fan_in).
 struct EnvRunner {
-  ckm_engine *e; const ckm_models *m; DomdefParams *p; const std::vector<PairWork> *pairs; DevBuf *dscratch;
+  ckm_engine *e; const ckm_models *m; DomdefParams *p; const std::vector<PairWork> *pairs;
   int64_t budget0;       // floats
-  int64_t cur_alloc;
   int nsm;
 };
 static int64_t env_scratch_budget() {
-  // fixed scratch budget (the cached pool is reused by every later search): 60% of the device shared by the live engines,
+  // fixed scratch budget (the EnvScratch workspace is reused by every later call): 60% of the device shared by the live engines,
   // at most 56 GiB each
   size_t free_b = 0, total_b = 0;
   cudaMemGetInfo(&free_b, &total_b);
@@ -369,7 +365,7 @@ static int64_t envelope_need(const ckm_models *m, const PairWork &pw, const Enve
   const int64_t width = vq ? 32 * vq : Mpad;
   return (vq ? 1 : 2) * (Ld + 1) * 3 * width + (Ld + 1) * 15 + 64;
 }
-static int run_envelope_waves(EnvRunner &R, std::vector<Envelope> &ev, DevBuf &d_ev, DevBuf &d_ord, bool leave_last) {
+static int run_envelope_waves(EnvRunner &R, std::vector<Envelope> &ev, Ws envs_key, Ws order_key, bool leave_last) {
   if (ev.empty()) return CKM_OK;
   ckm_engine *e = R.e; const ckm_models *m = R.m; DomdefParams &p = *R.p; const std::vector<PairWork> &pairs = *R.pairs;
   cudaStream_t st = e->stream;
@@ -383,19 +379,20 @@ static int run_envelope_waves(EnvRunner &R, std::vector<Envelope> &ev, DevBuf &d
     ecls[i] = (int8_t)cls_of(m->models[pw.model].M, p.use_blk != 0);
   }
   const int64_t budget = std::max<int64_t>(R.budget0, *std::max_element(need.begin(), need.end()));
-  if ((rc2 = d_ev.alloc(sizeof(Envelope) * ev.size())) || (rc2 = d_ord.alloc(sizeof(int32_t) * ev.size()))) return rc2;
+  Envelope *d_ev; int32_t *d_ord;
+  if ((rc2 = workspace(e, envs_key, sizeof(Envelope) * ev.size(), &d_ev)) || (rc2 = workspace(e, order_key, sizeof(int32_t) * ev.size(), &d_ord))) return rc2;
+  p.envs = d_ev; p.env_order = d_ord;
   std::vector<int32_t> eorder(ev.size());
   size_t w0 = 0;
   while (w0 < ev.size()) {
     size_t w1 = w0; int64_t tot = 0;
     while (w1 < ev.size() && (w1 == w0 || tot + need[w1] <= budget)) { ev[w1].scratch_off = tot; tot += need[w1]; ++w1; }
-    if (tot > R.cur_alloc) { if ((rc2 = R.dscratch->alloc(sizeof(float) * (size_t)tot))) return rc2; R.cur_alloc = tot; }
+    if ((rc2 = workspace(e, Ws::EnvScratch, sizeof(float) * (size_t)tot, &p.scratch))) return rc2;
     // this wave's envelopes grouped by class, largest first; one stream per class
     for (size_t i = w0; i < w1; ++i) eorder[i] = (int32_t)i;
     std::stable_sort(eorder.begin() + w0, eorder.begin() + w1, [&](int32_t a, int32_t b) { return ecls[a] != ecls[b] ? ecls[a] > ecls[b] : need[a] > need[b]; });
-    CKM_CUDA(cudaMemcpyAsync(d_ev.as<Envelope>() + w0, ev.data() + w0, sizeof(Envelope) * (w1 - w0), cudaMemcpyHostToDevice, st));
-    CKM_CUDA(cudaMemcpyAsync(d_ord.as<int32_t>() + w0, eorder.data() + w0, sizeof(int32_t) * (w1 - w0), cudaMemcpyHostToDevice, st));
-    p.envs = d_ev.as<Envelope>(); p.env_order = d_ord.as<int32_t>(); p.scratch = R.dscratch->as<float>();
+    CKM_CUDA(cudaMemcpyAsync(d_ev + w0, ev.data() + w0, sizeof(Envelope) * (w1 - w0), cudaMemcpyHostToDevice, st));
+    CKM_CUDA(cudaMemcpyAsync(d_ord + w0, eorder.data() + w0, sizeof(int32_t) * (w1 - w0), cudaMemcpyHostToDevice, st));
     if ((rc2 = fan_out(e))) return rc2;
     size_t b0 = w0;
     while (b0 < w1) {
@@ -442,9 +439,8 @@ static int do_search(ckm_engine *e, const ckm_models *m, const int32_t *model_id
   *hits_out = nullptr; *nhits_out = 0;
   const int ndb = (int)m->models.size();
   if (model_idx == nullptr && bin_model_offsets == nullptr) nmodels = ndb;
-  PoolScope pool_scope(e);
   ActiveMasks am; std::vector<int32_t> slot;
-  int rc = build_masks(m, db, model_idx, nmodels, bin_model_offsets, am, slot, st);
+  int rc = build_masks(e, m, db, model_idx, nmodels, bin_model_offsets, am, slot);
   if (rc) return rc;
   // query order per bin (for output ordering) and the number of pairs
   int64_t n_pairs = 0;
@@ -471,7 +467,7 @@ static int do_search(ckm_engine *e, const ckm_models *m, const int32_t *model_id
     if ((rc = run_stage1(e, m, db, am, std::max<int64_t>(n_pairs, 1), s1, nullptr, attempt))) return rc;
     if ((rc = run_stage2(e, m, db, am, s1, s2, nullptr, nullptr, nullptr, nullptr))) return rc;
     CKM_CUDA(cudaMemcpyAsync(ctr, e->d_counters, sizeof(ctr), cudaMemcpyDeviceToHost, st));
-    CKM_CUDA(cudaMemcpyAsync(&cells, s1.cells.p, sizeof(cells), cudaMemcpyDeviceToHost, st));
+    CKM_CUDA(cudaMemcpyAsync(&cells, s1.cells, sizeof(cells), cudaMemcpyDeviceToHost, st));
     CKM_CUDA(cudaStreamSynchronize(st));
     const bool over = ctr[CTR_CAND] > s1.cand_cap || ctr[CTR_MSV] > s1.pass_cap || ctr[CTR_BIAS] > s2.cap || ctr[CTR_VIT] > s2.cap || ctr[CTR_FWD] > s2.cap ||
                       ctr[CTR_VREDO] > s2.cap;
@@ -500,26 +496,25 @@ static int do_search(ckm_engine *e, const ckm_models *m, const int32_t *model_id
     pw.row_off = rows; rows += pw.L + 1;
   }
   const int nsm = e->prop.multiProcessorCount;
-  DevBuf dpairs, dxf, dxb, dvec, dregions, denvs, ddoms, dhits, dscratch, dtbl, dporder, deorder;
   std::vector<DomainOut> doms; std::vector<HitOut> hout((size_t)npairs);
   CKM_CUDA(cudaEventRecord(e->ev[6], st));
   tr.mark("pair list sorted");
   if (npairs > 0) {
     const size_t rws = (size_t)std::max<int64_t>(rows, 1);
-    if ((rc = dpairs.alloc(sizeof(PairWork) * pairs.size())) || (rc = dxf.alloc(sizeof(float) * rws * X_NX_HOST)) || (rc = dxb.alloc(sizeof(float) * rws * X_NX_HOST)) ||
-        (rc = dvec.alloc(sizeof(float) * rws * 4)) || (rc = dtbl.alloc(sizeof(float) * 16000))) return rc;
-    const int region_cap = npairs * 8 + 1024;
-    if ((rc = dregions.alloc(sizeof(Region) * (size_t)region_cap))) return rc;
-    CKM_CUDA(cudaMemcpyAsync(dpairs.p, pairs.data(), sizeof(PairWork) * pairs.size(), cudaMemcpyHostToDevice, st));
-    CKM_CUDA(cudaMemcpyAsync(dtbl.p, logsum_table().data(), sizeof(float) * 16000, cudaMemcpyHostToDevice, st));
-    CKM_CUDA(cudaMemsetAsync(e->d_counters + CTR_ENV, 0, sizeof(int32_t), st));
     DomdefParams p{};
+    PairWork *dpairs; float *dtbl;
+    const int region_cap = npairs * 8 + 1024;
+    if ((rc = workspace(e, Ws::Pairs, sizeof(PairWork) * pairs.size(), &dpairs)) || (rc = workspace(e, Ws::Xf, sizeof(float) * rws * X_NX_HOST, &p.xf)) ||
+        (rc = workspace(e, Ws::Xb, sizeof(float) * rws * X_NX_HOST, &p.xb)) || (rc = workspace(e, Ws::Vec, sizeof(float) * rws * 4, &p.btot)) ||
+        (rc = workspace(e, Ws::LogsumTbl, sizeof(float) * 16000, &dtbl)) || (rc = workspace(e, Ws::Regions, sizeof(Region) * (size_t)region_cap, &p.regions))) return rc;
+    CKM_CUDA(cudaMemcpyAsync(dpairs, pairs.data(), sizeof(PairWork) * pairs.size(), cudaMemcpyHostToDevice, st));
+    CKM_CUDA(cudaMemcpyAsync(dtbl, logsum_table().data(), sizeof(float) * 16000, cudaMemcpyHostToDevice, st));
+    CKM_CUDA(cudaMemsetAsync(e->d_counters + CTR_ENV, 0, sizeof(int32_t), st));
     p.res = db->d_res; p.off = db->d_off; p.nullsc = db->d_nullsc; p.ms = m->d_scalars; p.rfv = m->d_rfv; p.tfv = m->d_tfv;
-    p.pairs = dpairs.as<PairWork>(); p.npairs = npairs;
-    p.xf = dxf.as<float>(); p.xb = dxb.as<float>();
-    p.btot = dvec.as<float>(); p.etot = p.btot + rws; p.mocc = p.etot + rws; p.n2sc = p.mocc + rws;
-    p.regions = dregions.as<Region>(); p.region_count = e->d_counters + CTR_ENV; p.region_cap = region_cap;
-    p.logsum_tbl = dtbl.as<float>();
+    p.pairs = dpairs; p.npairs = npairs;
+    p.etot = p.btot + rws; p.mocc = p.etot + rws; p.n2sc = p.mocc + rws;
+    p.region_count = e->d_counters + CTR_ENV; p.region_cap = region_cap;
+    p.logsum_tbl = dtbl;
     p.row_elems = ((m->maxM + 31) / 32) * 32 + 64;
     p.tfb = m->d_tfb; p.rfb = m->d_rfb; p.use_blk = use_blocked_kernels() ? 1 : 0;
     {
@@ -528,9 +523,10 @@ static int do_search(ckm_engine *e, const ckm_models *m, const int32_t *model_id
       std::vector<int8_t> pcls((size_t)npairs);
       for (int i = 0; i < npairs; ++i) { order[i] = i; pcls[i] = (int8_t)cls_of(m->models[pairs[i].model].M, p.use_blk != 0); }
       std::stable_sort(order.begin(), order.end(), [&](int32_t a, int32_t b) { return pcls[a] != pcls[b] ? pcls[a] > pcls[b] : pairs[a].L > pairs[b].L; });
-      if ((rc = dporder.alloc(sizeof(int32_t) * order.size()))) return rc;
-      CKM_CUDA(cudaMemcpyAsync(dporder.p, order.data(), sizeof(int32_t) * order.size(), cudaMemcpyHostToDevice, st));
-      p.pair_order = dporder.as<int32_t>();
+      int32_t *dporder;
+      if ((rc = workspace(e, Ws::PairOrder, sizeof(int32_t) * order.size(), &dporder))) return rc;
+      CKM_CUDA(cudaMemcpyAsync(dporder, order.data(), sizeof(int32_t) * order.size(), cudaMemcpyHostToDevice, st));
+      p.pair_order = dporder;
       if ((rc = fan_out(e))) return rc;
       int b0 = 0;
       while (b0 < npairs) {
@@ -553,7 +549,7 @@ static int do_search(ckm_engine *e, const ckm_models *m, const int32_t *model_id
     CKM_CUDA(cudaStreamSynchronize(st));
     if (nreg > region_cap) { set_error("region queue overflow"); return CKM_ECAPACITY; }
     std::vector<Region> regs((size_t)nreg);
-    if (nreg) CKM_CUDA(cudaMemcpy(regs.data(), dregions.p, sizeof(Region) * regs.size(), cudaMemcpyDeviceToHost));
+    if (nreg) CKM_CUDA(cudaMemcpy(regs.data(), p.regions, sizeof(Region) * regs.size(), cudaMemcpyDeviceToHost));
     std::sort(regs.begin(), regs.end(), [](const Region &a, const Region &b) { return a.pair != b.pair ? a.pair < b.pair : a.i < b.i; });
     tr.mark("regions sorted");
     // Domain slots.  Regions are sorted by (pair, start), so a pair's slots are contiguous and in sequence order: one slot
@@ -566,7 +562,6 @@ static int do_search(ckm_engine *e, const ckm_models *m, const int32_t *model_id
     for (int r = 0; r < nreg; ++r) if (regs[r].multi) multi_idx.push_back(r);
     std::vector<EnsembleCaps> caps(multi_idx.size(), ENS_DEFAULT_CAPS);
     std::vector<int32_t> reg_slot((size_t)nreg);
-    DevBuf denvs2, deorder2;
     for (int pass = 0;; ++pass) {
     int32_t nslots = 0;
     for (auto &pw : pairs) { pw.ndom_slots = 0; pw.first_dom = 0; }
@@ -582,12 +577,12 @@ static int do_search(ckm_engine *e, const ckm_models *m, const int32_t *model_id
     for (int r = 0; r < nreg; ++r)
       if (!regs[r].multi) { Envelope en{}; en.pair = regs[r].pair; en.i = regs[r].i; en.j = regs[r].j; en.slot = reg_slot[r]; envs1.push_back(en); }
     if (nslots > 0) {
-      if ((rc = ddoms.alloc(sizeof(DomainOut) * (size_t)nslots)) || (rc = dhits.alloc(sizeof(HitOut) * pairs.size()))) return rc;
-      CKM_CUDA(cudaMemsetAsync(ddoms.p, 0, sizeof(DomainOut) * (size_t)nslots, st));
-      CKM_CUDA(cudaMemcpyAsync(dpairs.p, pairs.data(), sizeof(PairWork) * pairs.size(), cudaMemcpyHostToDevice, st));
-      p.doms = ddoms.as<DomainOut>();
-      EnvRunner R{e, m, &p, &pairs, &dscratch, env_scratch_budget(), 0, nsm};
-      auto run_env_batch = [&](std::vector<Envelope> &ev, DevBuf &d_ev, DevBuf &d_ord, bool leave_last) -> int { return run_envelope_waves(R, ev, d_ev, d_ord, leave_last); };
+      DomainOut *ddoms; HitOut *dhits;
+      if ((rc = workspace(e, Ws::Doms, sizeof(DomainOut) * (size_t)nslots, &ddoms)) || (rc = workspace(e, Ws::Hits, sizeof(HitOut) * pairs.size(), &dhits))) return rc;
+      CKM_CUDA(cudaMemsetAsync(ddoms, 0, sizeof(DomainOut) * (size_t)nslots, st));
+      CKM_CUDA(cudaMemcpyAsync(dpairs, pairs.data(), sizeof(PairWork) * pairs.size(), cudaMemcpyHostToDevice, st));
+      p.doms = ddoms;
+      EnvRunner R{e, m, &p, &pairs, env_scratch_budget(), nsm};
       // The trace ensemble of the multi-domain regions (one warp per region, latency-bound, its own stream) runs next to the
       // envelope kernels of the single-domain regions (class streams).  Next to them its dependent loads take 2-3x longer than
       // alone.  When the envelopes need more than one wave of scratch (large batches) it is queued FIRST and has all the waves to
@@ -606,7 +601,7 @@ static int do_search(ckm_engine *e, const ckm_models *m, const int32_t *model_id
         CKM_CUDA(cudaStreamWaitEvent(e->aux, e->fan_ev, 0));
         if ((rc = ensembles_launch(e, m, p, pairs, regs, multi_idx, caps, e->aux, &job))) { ensembles_abandon(job, e->aux); return rc; }
       }
-      if ((rc = run_env_batch(envs1, denvs, deorder, !multi_idx.empty()))) { if (job) ensembles_abandon(job, e->aux); return rc; }
+      if ((rc = run_envelope_waves(R, envs1, Ws::Envs1, Ws::EnvOrder1, !multi_idx.empty()))) { if (job) ensembles_abandon(job, e->aux); return rc; }
       tr.mark("envelope batch 1 launched");
       if (!multi_idx.empty()) {
         if (!ens_first) {
@@ -632,14 +627,14 @@ static int do_search(ckm_engine *e, const ckm_models *m, const int32_t *model_id
           int c = 0;
           for (Envelope en : multi_envs[mi]) { en.slot = reg_slot[multi_idx[mi]] + c++; envs2.push_back(en); }     // no more than the region's slots (ensembles_collect)
         }
-        if ((rc = run_env_batch(envs2, denvs2, deorder2, false))) return rc;
+        if ((rc = run_envelope_waves(R, envs2, Ws::Envs2, Ws::EnvOrder2, false))) return rc;
         tr.mark("envelope batch 2 done");
       }
-      p.hits = dhits.as<HitOut>();
+      p.hits = dhits;
       if ((rc = launch_scores(p, (npairs + 127) / 128, st))) return rc;
       e->stats.kernel_launches++;
-      CKM_CUDA(cudaMemcpyAsync(doms.data(), ddoms.p, sizeof(DomainOut) * doms.size(), cudaMemcpyDeviceToHost, st));
-      CKM_CUDA(cudaMemcpyAsync(hout.data(), dhits.p, sizeof(HitOut) * hout.size(), cudaMemcpyDeviceToHost, st));
+      CKM_CUDA(cudaMemcpyAsync(doms.data(), ddoms, sizeof(DomainOut) * doms.size(), cudaMemcpyDeviceToHost, st));
+      CKM_CUDA(cudaMemcpyAsync(hout.data(), dhits, sizeof(HitOut) * hout.size(), cudaMemcpyDeviceToHost, st));
       CKM_CUDA(cudaStreamSynchronize(st));
     } else {
       for (auto &h : hout) std::memset(&h, 0, sizeof(h));
@@ -781,22 +776,22 @@ int ckm_viterbi_scores(ckm_engine *e, const ckm_models *m, const int32_t *model_
   if (model_idx == nullptr) nmodels = ndb;
   const int64_t n = (int64_t)nmodels * db->nseq;
   if (n > ((int64_t)1 << 30)) { set_error("ckm_viterbi_scores: too many pairs for one call"); return CKM_ECAPACITY; }
-  PoolScope pool_scope(e);
   ActiveMasks am; std::vector<int32_t> slot;
-  int rc = build_masks(m, db, model_idx, nmodels, nullptr, am, slot, st);
+  int rc = build_masks(e, m, db, model_idx, nmodels, nullptr, am, slot);
   if (rc) return rc;
   std::vector<int32_t> slot_model((size_t)std::max(nmodels, 1));
   for (int i = 0; i < nmodels; ++i) slot_model[i] = model_idx ? model_idx[i] : i;
   const size_t nf = (size_t)std::max<int64_t>(n, 1);
-  DevBuf dsm, din, dout, dredo, dvit;
-  if ((rc = dsm.alloc(sizeof(int32_t) * slot_model.size())) || (rc = din.alloc(sizeof(Candidate) * nf)) || (rc = dout.alloc(sizeof(Candidate) * nf)) ||
-      (rc = dredo.alloc(sizeof(Candidate) * nf)) || (rc = dvit.alloc(sizeof(float) * nf))) return rc;
-  CKM_CUDA(cudaMemcpyAsync(dsm.p, slot_model.data(), sizeof(int32_t) * slot_model.size(), cudaMemcpyHostToDevice, st));
+  int32_t *dsm; Candidate *din, *dout, *dredo; float *dvit;
+  if ((rc = workspace(e, Ws::SlotModel, sizeof(int32_t) * slot_model.size(), &dsm)) || (rc = workspace(e, Ws::ListA, sizeof(Candidate) * nf, &din)) ||
+      (rc = workspace(e, Ws::ListB, sizeof(Candidate) * nf, &dout)) || (rc = workspace(e, Ws::Redo, sizeof(Candidate) * nf, &dredo)) ||
+      (rc = workspace(e, Ws::DenseVit, sizeof(float) * nf, &dvit))) return rc;
+  CKM_CUDA(cudaMemcpyAsync(dsm, slot_model.data(), sizeof(int32_t) * slot_model.size(), cudaMemcpyHostToDevice, st));
   CKM_CUDA(cudaMemsetAsync(e->d_counters, 0, CTR_N * sizeof(int32_t), st));
-  CKM_CUDA(cudaMemsetAsync(dvit.p, 0xff, sizeof(float) * nf, st));
+  CKM_CUDA(cudaMemsetAsync(dvit, 0xff, sizeof(float) * nf, st));
   std::memset(&e->stats, 0, sizeof(e->stats));
   if (n > 0) {
-    if ((rc = launch_all_pairs(din.as<Candidate>(), e->d_counters + CTR_BIAS, dsm.as<int32_t>(), nmodels, db->nseq, st))) return rc;
+    if ((rc = launch_all_pairs(din, e->d_counters + CTR_BIAS, dsm, nmodels, db->nseq, st))) return rc;
     const int nsm = e->prop.multiProcessorCount;
     FilterParams p{};
     p.res = db->d_res; p.off = db->d_off; p.len = db->d_len; p.lenA = db->d_lenA; p.lenB = db->d_lenB; p.tmove_w = db->d_tmove_w;
@@ -804,16 +799,16 @@ int ckm_viterbi_scores(ckm_engine *e, const ckm_models *m, const int32_t *model_
     p.twb = m->d_twb; p.rwb = m->d_rwb; p.tfb = m->d_tfb; p.rfb = m->d_rfb; p.twp = m->d_twp; p.rwp = m->d_rwp;
     p.row_elems = ((m->maxM + 31) / 32) * 32 + 64;
     p.F1 = 0.02; p.F2 = 1e-3; p.F3 = 1e-5; p.use_blk = (mode == 2) ? 0 : 1;      // mode 2: every pair through the chunked shared-memory kernel
-    p.dense_vit = dvit.as<float>(); p.model_slot = am.model_slot.as<int32_t>(); p.nseq = db->nseq;
-    p.redo = dredo.as<Candidate>(); p.redo_count = e->d_counters + CTR_VREDO; p.redo_cap = (int32_t)nf;
-    p.in = din.as<Candidate>(); p.in_count = e->d_counters + CTR_BIAS; p.in_cap = (int32_t)nf;
-    p.out = dout.as<Candidate>(); p.out_count = e->d_counters + CTR_VIT; p.out_cap = (int32_t)nf;
+    p.dense_vit = dvit; p.model_slot = am.model_slot; p.nseq = db->nseq;
+    p.redo = dredo; p.redo_count = e->d_counters + CTR_VREDO; p.redo_cap = (int32_t)nf;
+    p.in = din; p.in_count = e->d_counters + CTR_BIAS; p.in_cap = (int32_t)nf;
+    p.out = dout; p.out_count = e->d_counters + CTR_VIT; p.out_cap = (int32_t)nf;
     if (mode == 0) {
       p.vit_work = e->d_counters + CTR_VWORK;
       if ((rc = fan_out(e))) return rc;
       for (int c = 0; c < N_BLK_CLASSES; ++c) if ((rc = launch_vitp(p, c, nsm * 8, e->cls[c]))) return rc;
       if ((rc = fan_in(e))) return rc;
-      p.in = dredo.as<Candidate>(); p.in_count = e->d_counters + CTR_VREDO;
+      p.in = dredo; p.in_count = e->d_counters + CTR_VREDO;
     }
     if ((rc = fan_out(e))) return rc;
     if (p.use_blk) { for (int c = 0; c < N_BLK_CLASSES; ++c) if ((rc = launch_vit2(p, c, nsm * 8, e->cls[c]))) return rc; }
@@ -822,7 +817,7 @@ int ckm_viterbi_scores(ckm_engine *e, const ckm_models *m, const int32_t *model_
   }
   int32_t ctr[CTR_N];
   CKM_CUDA(cudaMemcpyAsync(ctr, e->d_counters, sizeof(ctr), cudaMemcpyDeviceToHost, st));
-  CKM_CUDA(cudaMemcpyAsync(vit_out, dvit.p, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, st));
+  CKM_CUDA(cudaMemcpyAsync(vit_out, dvit, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, st));
   CKM_CUDA(cudaStreamSynchronize(st));
   e->stats.n_pairs = n; e->stats.n_past_bias = ctr[CTR_BIAS]; e->stats.n_past_vit = ctr[CTR_VIT]; e->stats.n_vit_redo = ctr[CTR_VREDO];
   return CKM_OK;
@@ -833,22 +828,21 @@ int ckm_msv_scores(ckm_engine *e, const ckm_models *m, const int32_t *model_idx,
   if (!e || !m || !db || !xj_out) { set_error("ckm_msv_scores: bad argument"); return CKM_EINVAL; }
   cudaSetDevice(e->device);
   if (model_idx == nullptr) nmodels = (int32_t)m->models.size();
-  PoolScope pool_scope(e);
   ActiveMasks am; std::vector<int32_t> slot;
-  int rc = build_masks(m, db, model_idx, nmodels, nullptr, am, slot, e->stream);
+  int rc = build_masks(e, m, db, model_idx, nmodels, nullptr, am, slot);
   if (rc) return rc;
   const int64_t n = (int64_t)nmodels * db->nseq;
-  DevBuf dense;
-  if ((rc = dense.alloc(sizeof(int32_t) * (size_t)std::max<int64_t>(n, 1)))) return rc;
-  CKM_CUDA(cudaMemsetAsync(dense.p, 0xff, sizeof(int32_t) * (size_t)n, e->stream));
+  int32_t *dense;
+  if ((rc = workspace(e, Ws::DenseXj, sizeof(int32_t) * (size_t)std::max<int64_t>(n, 1), &dense))) return rc;
+  CKM_CUDA(cudaMemsetAsync(dense, 0xff, sizeof(int32_t) * (size_t)n, e->stream));
   Stage1 s1;
   std::memset(&e->stats, 0, sizeof(e->stats));
-  if ((rc = run_stage1(e, m, db, am, n, s1, dense.as<int32_t>()))) return rc;
+  if ((rc = run_stage1(e, m, db, am, n, s1, dense))) return rc;
   int32_t ctr[CTR_N];
   CKM_CUDA(cudaMemcpyAsync(ctr, e->d_counters, sizeof(ctr), cudaMemcpyDeviceToHost, e->stream));
   unsigned long long cells = 0;
-  CKM_CUDA(cudaMemcpyAsync(&cells, s1.cells.p, sizeof(cells), cudaMemcpyDeviceToHost, e->stream));
-  CKM_CUDA(cudaMemcpyAsync(xj_out, dense.p, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
+  CKM_CUDA(cudaMemcpyAsync(&cells, s1.cells, sizeof(cells), cudaMemcpyDeviceToHost, e->stream));
+  CKM_CUDA(cudaMemcpyAsync(xj_out, dense, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, e->stream));
   CKM_CUDA(cudaStreamSynchronize(e->stream));
   if (ctr[CTR_CAND] > s1.cand_cap || ctr[CTR_MSV] > s1.pass_cap) { set_error("candidate queue overflow"); return CKM_ECAPACITY; }
   e->stats.n_pairs = n; e->stats.n_cells = (int64_t)cells;
@@ -870,30 +864,27 @@ namespace ckm {
 static int align_pass(ckm_engine *e, const ckm_models *m, const ckm_seqdb *db, std::vector<PairWork> &pairs, std::vector<Envelope> &envs,
                       int64_t rows, std::vector<int32_t> &trace, std::vector<DomainOut> &doms) {
   cudaStream_t st = e->stream;
-  PoolScope pool_scope(e);
   const int nsm = e->prop.multiProcessorCount;
-  DevBuf dpairs, dn2, dtrace, ddoms, dscratch, denvs, deorder;
+  DomdefParams p{};
+  PairWork *dpairs;
   int rc;
   const size_t rws = (size_t)rows;
-  if ((rc = dpairs.alloc(sizeof(PairWork) * pairs.size())) || (rc = dn2.alloc(sizeof(float) * rws)) || (rc = dtrace.alloc(sizeof(int32_t) * rws)) ||
-      (rc = ddoms.alloc(sizeof(DomainOut) * pairs.size()))) return rc;
-  CKM_CUDA(cudaMemcpyAsync(dpairs.p, pairs.data(), sizeof(PairWork) * pairs.size(), cudaMemcpyHostToDevice, st));
-  CKM_CUDA(cudaMemsetAsync(dn2.p, 0, sizeof(float) * rws, st));
-  CKM_CUDA(cudaMemsetAsync(dtrace.p, 0, sizeof(int32_t) * rws, st));
-  CKM_CUDA(cudaMemsetAsync(ddoms.p, 0, sizeof(DomainOut) * pairs.size(), st));
-  DomdefParams p{};
+  if ((rc = workspace(e, Ws::Pairs, sizeof(PairWork) * pairs.size(), &dpairs)) || (rc = workspace(e, Ws::Vec, sizeof(float) * rws, &p.n2sc)) ||
+      (rc = workspace(e, Ws::AlignTrace, sizeof(int32_t) * rws, &p.trace)) || (rc = workspace(e, Ws::Doms, sizeof(DomainOut) * pairs.size(), &p.doms))) return rc;
+  CKM_CUDA(cudaMemcpyAsync(dpairs, pairs.data(), sizeof(PairWork) * pairs.size(), cudaMemcpyHostToDevice, st));
+  CKM_CUDA(cudaMemsetAsync(p.n2sc, 0, sizeof(float) * rws, st));
+  CKM_CUDA(cudaMemsetAsync(p.trace, 0, sizeof(int32_t) * rws, st));
+  CKM_CUDA(cudaMemsetAsync(p.doms, 0, sizeof(DomainOut) * pairs.size(), st));
   p.res = db->d_res; p.off = db->d_off; p.nullsc = db->d_nullsc; p.ms = m->d_scalars; p.rfv = m->d_rfv; p.tfv = m->d_tfv;
-  p.pairs = dpairs.as<PairWork>(); p.npairs = (int32_t)pairs.size();
-  p.n2sc = dn2.as<float>(); p.trace = dtrace.as<int32_t>();
-  p.doms = ddoms.as<DomainOut>();
+  p.pairs = dpairs; p.npairs = (int32_t)pairs.size();
   p.row_elems = ((m->maxM + 31) / 32) * 32 + 64;
   p.tfb = m->d_tfb; p.rfb = m->d_rfb; p.use_blk = use_blocked_kernels() ? 1 : 0;
-  EnvRunner R{e, m, &p, &pairs, &dscratch, env_scratch_budget(), 0, nsm};
-  if ((rc = run_envelope_waves(R, envs, denvs, deorder, false))) return rc;
+  EnvRunner R{e, m, &p, &pairs, env_scratch_budget(), nsm};
+  if ((rc = run_envelope_waves(R, envs, Ws::Envs1, Ws::EnvOrder1, false))) return rc;
   trace.resize(rws);
   doms.resize(pairs.size());
-  CKM_CUDA(cudaMemcpyAsync(trace.data(), dtrace.p, sizeof(int32_t) * rws, cudaMemcpyDeviceToHost, st));
-  CKM_CUDA(cudaMemcpyAsync(doms.data(), ddoms.p, sizeof(DomainOut) * doms.size(), cudaMemcpyDeviceToHost, st));
+  CKM_CUDA(cudaMemcpyAsync(trace.data(), p.trace, sizeof(int32_t) * rws, cudaMemcpyDeviceToHost, st));
+  CKM_CUDA(cudaMemcpyAsync(doms.data(), p.doms, sizeof(DomainOut) * doms.size(), cudaMemcpyDeviceToHost, st));
   CKM_CUDA(cudaStreamSynchronize(st));
   return CKM_OK;
 }

@@ -102,6 +102,12 @@ class Engine:
         check(_lib.lib().ckm_last_stats(self._h, C.byref(s)))
         return s
 
+    def workspace_bytes(self):
+        """Device bytes the engine keeps between calls as workspaces (ckm_workspace_bytes)."""
+        n = C.c_int64()
+        check(_lib.lib().ckm_workspace_bytes(self._h, C.byref(n)))
+        return n.value
+
     def msv_scores(self, models, db, model_idx=None):
         """Dense [nmodels, nseq] int32: exact MSV xJ byte for SSV candidates (256 = overflow), -1 otherwise."""
         nm = models.n if model_idx is None else len(model_idx)

@@ -163,6 +163,10 @@ void ckm_hits_free(ckm_hit *hits);
  * insert state -k, 0 unaligned flank.  oasc_out[nseq] (optional): the optimal-accuracy score, 0 if no alignment exists. ---- */
 int  ckm_align(ckm_engine *e, const ckm_models *m, int32_t model, const ckm_seqdb *db, int32_t *state_out, float *oasc_out);
 int  ckm_last_stats(const ckm_engine *e, ckm_stats *out);
+/* device bytes the engine keeps between calls as workspaces (one grow-only buffer per role, slack included); models, sequence
+ * databases and the stream-ordered pool are not counted.  It follows from the largest inputs the engine has seen, not from
+ * the order of its calls. */
+int  ckm_workspace_bytes(const ckm_engine *e, int64_t *bytes_out);
 
 /* stage-level entry points for parity tests (device arrays come back to host buffers the caller owns) */
 int  ckm_msv_scores(ckm_engine *e, const ckm_models *m, const int32_t *model_idx, int32_t nmodels,
@@ -227,8 +231,8 @@ typedef struct {
 
 /* hits: domtblout rows grouped by bin (ascending) and, inside a bin, by query (rows of one query contiguous, in file
  * order).  `model` and `seq` index the caller's model table (nmodels entries) and sequence table (nseq entries).
- * When the device has no room left for the reduction, the engine's cached search workspaces are freed and the call is
- * tried once more; the engine's next search allocates them again. */
+ * When the device has no room left for the reduction, the engine's workspaces (ckm_workspace_bytes) are freed and the call
+ * is tried once more; the engine's next call allocates what it needs again. */
 int  ckm_reduce(ckm_engine *e, int32_t nmodels, int32_t nseq, int32_t nbins, const ckm_hit *hits, int64_t nhits,
                 const ckm_reduce_opts *opts, const ckm_reduce_meta *meta,
                 ckm_qa_row **qa_out, int32_t *nqa_out, ckm_marker_hit **mh_out, int64_t *nmh_out);
