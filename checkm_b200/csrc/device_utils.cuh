@@ -50,6 +50,38 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
       : "memory");
 }
 
+// ---- tensor memory (tcgen05; SASS: UTCATOMSWS, LDTM, STTM).  Addresses are (lane << 16) | column; a warp may touch only the
+// 32 lanes of its sub-partition, 32 * (warp % 4) onwards.  alloc / relinquish / dealloc are whole-warp instructions. ----
+__device__ __forceinline__ void tmem_alloc(uint32_t *dst_smem, uint32_t ncols) {
+  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(ncols) : "memory");
+}
+// gives the columns back and gives up the CTA's right to allocate again
+__device__ __forceinline__ void tmem_release(uint32_t taddr, uint32_t ncols) {
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+__device__ __forceinline__ void tmem_fence_before_sync() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tmem_fence_after_sync() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+// 16 consecutive columns of the calling thread's lane; the registers are valid only after tmem_wait_ld()
+__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
+                 "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+               : "r"(taddr));
+}
+__device__ __forceinline__ void tmem_wait_ld(uint32_t (&r)[16]) {
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+  for (int j = 0; j < 16; ++j) asm volatile("" : "+r"(r[j]));     // no use of r may be scheduled above the wait
+}
+__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
+               ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]),
+                 "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
+               : "memory");
+}
+__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
 // ---- warp reductions ----
 __device__ __forceinline__ int warp_max_int(int v) {
 #pragma unroll

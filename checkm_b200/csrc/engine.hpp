@@ -22,11 +22,19 @@ constexpr int MAX_MODEL_M = 4608;
 // J = 32 tiles keep the first two quads (words 0..7 of every lane) as int8 pairs in ONE 16-byte chunk per lane
 // (gains clamped at -128, exact while u < 128; the kernel flags any slot that reaches 127): 7 instead of 8 LDS.128 per
 // row, the sign-extending unpack costs one PRMT per word on the ALU pipe, which has the headroom.
+// TMEM-assisted J = 32 tiles (the default, ckm_models::ssv_tmem) keep every word as int16 instead: the kernel copies words
+// 0..SSV_TMEM_WORDS-1 of every lane and residue into tensor memory once per tile, and a row then reads them with one
+// tcgen05.ld next to 4 LDS.128 for the rest (tensor memory feeds registers without using the shared-memory pipe).
 // ------------------------------------------------------------------------------------------------
-constexpr int SSV_I8_WORDS = 8;       // words per lane stored as int8 pairs in J = 32 tiles
-__host__ __device__ constexpr int ssv_row_bytes(int J) { return (J == 32) ? 128 * J - 16 * 32 * (SSV_I8_WORDS / 4 - 1) : 128 * J; }
-__host__ __device__ constexpr int ssv_table_bytes(int J) { return KPAD * ssv_row_bytes(J); }
-__host__ __device__ constexpr int ssv_block_bytes(int J) { return ssv_table_bytes(J) + 768; }
+constexpr int SSV_I8_WORDS = 8;       // words per lane stored as int8 pairs in J = 32 tiles without tensor memory
+constexpr int SSV_TMEM_WORDS = 16;    // words per lane read from tensor memory in TMEM-assisted J = 32 tiles
+static_assert(KPAD * SSV_TMEM_WORDS <= 512, "a TMEM-assisted tile must fit the 512 tensor-memory columns of an SM");
+__host__ __device__ constexpr bool ssv_int8_chunk(int J, bool tmem) { return J == 32 && !tmem; }
+__host__ __device__ constexpr int ssv_row_bytes(int J, bool tmem) {
+  return ssv_int8_chunk(J, tmem) ? 128 * J - 16 * 32 * (SSV_I8_WORDS / 4 - 1) : 128 * J;
+}
+__host__ __device__ constexpr int ssv_table_bytes(int J, bool tmem) { return KPAD * ssv_row_bytes(J, tmem); }
+__host__ __device__ constexpr int ssv_block_bytes(int J, bool tmem) { return ssv_table_bytes(J, tmem) + 768; }
 struct TileModel {       // one model (or one 1024-cell chunk of a long model) inside a tile
   int32_t model;         // database index
   int32_t slot0, nslots;
@@ -126,6 +134,7 @@ struct ckm_models {
   std::vector<int32_t>        chain_first_tile;   // per chain
   std::vector<int32_t>        chain_ntiles;
   std::vector<int32_t>        ssv_bypass;         // models without SSV tiles (chain larger than shared memory): all their pairs are MSV candidates
+  bool            ssv_tmem = true;                // J = 32 tiles use the TMEM-assisted layout (CKM_SSV_TMEM=0 at load: the int8-chunk layout)
   int32_t        *d_ssv_bypass = nullptr;
   ckm::TileDesc  *d_tiles = nullptr;
   ckm::TileModel *d_tile_models = nullptr;

@@ -23,21 +23,25 @@ namespace ckm {
 // SSV pre-filter
 // ------------------------------------------------------------------------------------------------
 
-template <int J> __host__ __device__ constexpr int tile_table_bytes() { return ssv_table_bytes(J); }
-template <int J> __host__ __device__ constexpr int tile_block_bytes() { return ssv_block_bytes(J); }
+template <int J, bool TM> __host__ __device__ constexpr int tile_table_bytes() { return ssv_table_bytes(J, TM); }
+template <int J, bool TM> __host__ __device__ constexpr int tile_block_bytes() { return ssv_block_bytes(J, TM); }
+constexpr uint32_t SSV_TMEM_COLS = 512;   // a TMEM-assisted CTA owns all of the SM's tensor memory (one CTA per SM)
 
-
-template <int J>
-__device__ __forceinline__ void ssv_rows(const uint8_t *__restrict__ res, int L, uint32_t tile_smem, int lane, uint32_t sel,
-                                         const int16_t *bnd_in, int16_t *bnd_out, uint32_t (&u)[J], uint32_t &xE) {
+// TM: words 0..SSV_TMEM_WORDS-1 of every row come from tensor memory at column x * SSV_TMEM_WORDS of lane tmem_lane
+template <int J, bool TM>
+__device__ __forceinline__ void ssv_rows(const uint8_t *__restrict__ res, int L, uint32_t tile_smem, uint32_t tmem_lane, int lane,
+                                         uint32_t sel, const int16_t *bnd_in, int16_t *bnd_out, uint32_t (&u)[J], uint32_t &xE) {
   constexpr int G = J / 4;
   const uint4 *rp = reinterpret_cast<const uint4 *>(res);
   const uint32_t lane_off = tile_smem + lane * 16;
-  constexpr bool I8 = (J == 32);                       // words 0..7 of every lane come as int8 pairs in one 16-byte chunk
-  constexpr int G0 = I8 ? SSV_I8_WORDS / 4 : 0;       // int16 quads start here
+  constexpr bool I8 = ssv_int8_chunk(J, TM);          // words 0..7 of every lane come as int8 pairs in one 16-byte chunk
+  constexpr int G0 = I8 ? SSV_I8_WORDS / 4 : TM ? SSV_TMEM_WORDS / 4 : 0;       // int16 quads read from shared memory start here
+  static_assert(!TM || J == 32, "TMEM-assisted tiles are J = 32 tiles");
   auto do_row = [&](uint32_t x, int i) {
-    const uint32_t row = lane_off + x * ssv_row_bytes(J);
+    const uint32_t row = lane_off + x * ssv_row_bytes(J, TM);
     uint4 e[G];
+    uint32_t t[TM ? SSV_TMEM_WORDS : 1];
+    if constexpr (TM) tmem_ld16(tmem_lane + x * SSV_TMEM_WORDS, t);
     if (I8) {
       const uint4 c = lds128(row);
       const uint32_t cw[4] = {c.x, c.y, c.z, c.w};
@@ -46,6 +50,11 @@ __device__ __forceinline__ void ssv_rows(const uint8_t *__restrict__ res, int L,
     }
 #pragma unroll
     for (int g = G0; g < G; ++g) e[g] = lds128(row + (g - (I8 ? G0 - 1 : 0)) * 512);
+    if constexpr (TM) {
+      tmem_wait_ld(t);
+#pragma unroll
+      for (int q = 0; q < SSV_TMEM_WORDS; ++q) (&e[q >> 2].x)[q & 3] = t[q];
+    }
     uint32_t bndw = 0;
     if (bnd_in != nullptr) bndw = (i > 0) ? (uint32_t)(uint16_t)bnd_in[i - 1] : 0u;      // chained tile: cell 0 continues the previous chunk's last cell
     const uint32_t sh = __shfl_sync(0xffffffffu, u[J - 1], (lane + 31) & 31);
@@ -78,19 +87,30 @@ __device__ __forceinline__ void ssv_rows(const uint8_t *__restrict__ res, int L,
   }
 }
 
-template <int J>
+// TM: a TMEM-assisted J = 32 tile (every group holds one tile, models.cu).  Warp w reads the tensor-memory lanes of its
+// sub-partition, 32 * (w % 4) + lane, so each of the four lane quarters holds its own copy of the tile's TMEM words.
+template <int J, bool TM>
 __global__ void __launch_bounds__(SSV_WARPS * 32, 1) ssv_kernel(SsvParams p) {
+  static_assert(!TM || SSV_WARPS % 4 == 0, "every sub-partition needs warps to fill its copy of the TMEM words");
   extern __shared__ __align__(128) uint8_t smem[];
   __shared__ __align__(8) uint64_t bar;
   __shared__ int s_unit, s_item;
+  __shared__ uint32_t s_tmem;
   __shared__ int16_t su[SSV_WARPS][64];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const uint32_t smem_base = smem_u32(smem);
   const uint32_t sel = (lane == 0) ? 0x1054u : 0x3210u;
-  constexpr int TB = tile_block_bytes<J>();
-  constexpr int I8CAP = (J == 32) ? 127 : 32767;
-  if (tid == 0) { mbar_init(&bar, 1); fence_mbar_init(); }
+  constexpr int TB = tile_block_bytes<J, TM>();
+  // gains clamped to int8 are exact only while u < 128, so a slot that reaches 127 is flagged as a candidate
+  constexpr int I8CAP = ssv_int8_chunk(J, TM) ? 127 : 32767;
+  if (warp == 0) {
+    if (TM) tmem_alloc(&s_tmem, SSV_TMEM_COLS);
+    if (lane == 0) { mbar_init(&bar, 1); fence_mbar_init(); }
+  }
+  if (TM) tmem_fence_before_sync();
   __syncthreads();
+  if (TM) tmem_fence_after_sync();
+  const uint32_t tmem_lane = TM ? s_tmem + ((uint32_t)(32 * (warp & 3)) << 16) : 0u;
   uint32_t phase = 0;
   int cur_group = -1;
   unsigned long long my_cells = 0;
@@ -98,7 +118,9 @@ __global__ void __launch_bounds__(SSV_WARPS * 32, 1) ssv_kernel(SsvParams p) {
   int16_t *bndB = p.bnd ? bndA + p.bnd_stride : nullptr;
 
   while (true) {
+    if (TM) tmem_fence_before_sync();
     __syncthreads();                       // everybody is done with the previous unit (tables + s_item)
+    if (TM) tmem_fence_after_sync();
     if (tid == 0) { s_unit = atomicAdd(p.unit_counter, 1); s_item = 0; }
     __syncthreads();
     const int unit = s_unit;
@@ -115,6 +137,22 @@ __global__ void __launch_bounds__(SSV_WARPS * 32, 1) ssv_kernel(SsvParams p) {
       }
       mbar_wait(&bar, phase);
       phase ^= 1;
+      if constexpr (TM) {                  // copy words 0..SSV_TMEM_WORDS-1 of every row into this sub-partition's TMEM lanes
+        for (int x = warp >> 2; x < KPAD; x += SSV_WARPS / 4) {
+          const uint32_t row = smem_base + lane * 16 + x * ssv_row_bytes(J, TM);
+          uint32_t w[SSV_TMEM_WORDS];
+#pragma unroll
+          for (int g = 0; g < SSV_TMEM_WORDS / 4; ++g) {
+            const uint4 v = lds128(row + g * 512);
+            w[4 * g] = v.x; w[4 * g + 1] = v.y; w[4 * g + 2] = v.z; w[4 * g + 3] = v.w;
+          }
+          tmem_st16(tmem_lane + x * SSV_TMEM_WORDS, w);
+        }
+        tmem_wait_st();
+        tmem_fence_before_sync();
+        __syncthreads();
+        tmem_fence_after_sync();
+      }
     }
     const int s_begin = chunk * p.seq_chunk;
     const int s_count = min(p.seq_chunk, p.nseq - s_begin);
@@ -128,7 +166,7 @@ __global__ void __launch_bounds__(SSV_WARPS * 32, 1) ssv_kernel(SsvParams p) {
       const int chain = grp.first_chain + it % grp.nchains;
       const int L = p.len[s];
       if (L == 0) continue;
-      const int t0 = p.chain_first_tile[chain], nt = p.chain_ntiles[chain];
+      const int t0 = p.chain_first_tile[chain], nt = TM ? 1 : p.chain_ntiles[chain];     // J = 32 tiles are never chained
       const int sbin = p.bin[s];
       if (p.tile_active != nullptr && !p.tile_active[(int64_t)sbin * p.ntiles + t0]) continue;
       const uint8_t *res = p.res + p.off[s];
@@ -145,15 +183,14 @@ __global__ void __launch_bounds__(SSV_WARPS * 32, 1) ssv_kernel(SsvParams p) {
         uint32_t xE = 0u;
         const int16_t *bin_ = (nt > 1 && tt > 0) ? ((tt & 1) ? bndA : bndB) : nullptr;
         int16_t *bout = (nt > 1 && tt + 1 < nt) ? ((tt & 1) ? bndB : bndA) : nullptr;
-        ssv_rows<J>(res, L, tsm, lane, sel, bin_, bout, u, xE);
+        ssv_rows<J, TM>(res, L, tsm, tmem_lane, lane, sel, bin_, bout, u, xE);
         my_cells += (unsigned long long)L * (2 * J);
         // ---- epilogue: does any slot reach the candidate bound? ----
-        const uint8_t *meta = smem + tl * TB + tile_table_bytes<J>();
+        const uint8_t *meta = smem + tl * TB + tile_table_bytes<J, TM>();
         const float *A = reinterpret_cast<const float *>(meta);
         const int32_t *F = reinterpret_cast<const int32_t *>(meta + 256);
         const int32_t *SM = reinterpret_cast<const int32_t *>(meta + 512);
         const int ulo = (int)(int16_t)(xE & 0xffffu), uhi = (int)(int16_t)(xE >> 16);
-        // (J = 32 tiles carry int8 gains clamped at -128: exact while u < 128, so a slot that reached 127 is forwarded too)
         const int thr_lo = min(min((int)floorf(A[lane] + Bs) - 1, F[lane] + tjb), I8CAP);
         const int thr_hi = min(min((int)floorf(A[32 + lane] + Bs) - 1, F[32 + lane] + tjb), I8CAP);
         const bool c_lo = (SM[lane] >= 0) && (ulo >= thr_lo);
@@ -216,44 +253,36 @@ __global__ void __launch_bounds__(SSV_WARPS * 32, 1) ssv_kernel(SsvParams p) {
       }
     }
   }
+  if (TM && warp == 0) tmem_release(s_tmem, SSV_TMEM_COLS);     // the loop's last barrier ordered every warp's TMEM reads before this
   // statistics
   my_cells = warp_sum_ull(my_cells);
   if (lane == 0 && p.cells != nullptr) atomicAdd(p.cells, my_cells);
 }
 
-template __global__ void ssv_kernel<4>(SsvParams);
-template __global__ void ssv_kernel<8>(SsvParams);
-template __global__ void ssv_kernel<16>(SsvParams);
-template __global__ void ssv_kernel<32>(SsvParams);
+template __global__ void ssv_kernel<4, false>(SsvParams);
+template __global__ void ssv_kernel<8, false>(SsvParams);
+template __global__ void ssv_kernel<16, false>(SsvParams);
+template __global__ void ssv_kernel<32, false>(SsvParams);
+template __global__ void ssv_kernel<32, true>(SsvParams);
 
-int launch_ssv(int J, const SsvParams &p, int grid, size_t smem_bytes, cudaStream_t stream) {
-  cudaError_t e;
-  switch (J) {
-    case 4:
-      e = cudaFuncSetAttribute(ssv_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
-      if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(ssv<4>)");
-      ssv_kernel<4><<<grid, SSV_WARPS * 32, smem_bytes, stream>>>(p);
-      break;
-    case 8:
-      e = cudaFuncSetAttribute(ssv_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
-      if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(ssv<8>)");
-      ssv_kernel<8><<<grid, SSV_WARPS * 32, smem_bytes, stream>>>(p);
-      break;
-    case 16:
-      e = cudaFuncSetAttribute(ssv_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
-      if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(ssv<16>)");
-      ssv_kernel<16><<<grid, SSV_WARPS * 32, smem_bytes, stream>>>(p);
-      break;
-    case 32:
-      e = cudaFuncSetAttribute(ssv_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
-      if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(ssv<32>)");
-      ssv_kernel<32><<<grid, SSV_WARPS * 32, smem_bytes, stream>>>(p);
-      break;
-    default: set_error("unsupported tile width"); return CKM_EINVAL;
-  }
+template <int J, bool TM>
+static int launch_ssv_t(const SsvParams &p, int grid, size_t smem_bytes, cudaStream_t stream) {
+  cudaError_t e = cudaFuncSetAttribute(ssv_kernel<J, TM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(ssv_kernel)");
+  ssv_kernel<J, TM><<<grid, SSV_WARPS * 32, smem_bytes, stream>>>(p);
   e = cudaGetLastError();
   if (e != cudaSuccess) return cuda_fail(e, "ssv_kernel launch");
   return CKM_OK;
+}
+
+int launch_ssv(int J, bool tmem, const SsvParams &p, int grid, size_t smem_bytes, cudaStream_t stream) {
+  switch (J) {
+    case 4: return launch_ssv_t<4, false>(p, grid, smem_bytes, stream);
+    case 8: return launch_ssv_t<8, false>(p, grid, smem_bytes, stream);
+    case 16: return launch_ssv_t<16, false>(p, grid, smem_bytes, stream);
+    case 32: return tmem ? launch_ssv_t<32, true>(p, grid, smem_bytes, stream) : launch_ssv_t<32, false>(p, grid, smem_bytes, stream);
+    default: set_error("unsupported tile width"); return CKM_EINVAL;
+  }
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -27,8 +27,6 @@ static int upload(T **dptr, const std::vector<T> &h) {
   return CKM_OK;
 }
 
-static int tile_block_bytes_host(int J) { return ssv_block_bytes(J); }
-
 // Packs the models into SSV tiles (see engine.hpp) and builds the int16 emission-delta tables.
 static void build_tiles(ckm_models &db, std::vector<uint8_t> &blob) {
   const int n = (int)db.models.size();
@@ -38,6 +36,9 @@ static void build_tiles(ckm_models &db, std::vector<uint8_t> &blob) {
   int fixedJ = 32;
   if (pol != nullptr) { if (!std::strcmp(pol, "auto")) fixedJ = 0; else fixedJ = std::atoi(pol); }
   if (fixedJ != 0 && fixedJ != 4 && fixedJ != 8 && fixedJ != 16 && fixedJ != 32) fixedJ = 32;
+  // J = 32 table layout: TMEM-assisted (default) or with the int8 chunk (CKM_SSV_TMEM=0, kept as the cross-check)
+  { const char *v = std::getenv("CKM_SSV_TMEM"); db.ssv_tmem = !(v != nullptr && v[0] == '0'); }
+  const bool tmem = db.ssv_tmem;
   std::vector<Item> cls[3], longm;
   int Js[3] = {4, 8, 16};
   int chainJ = 16;
@@ -78,7 +79,7 @@ static void build_tiles(ckm_models &db, std::vector<uint8_t> &blob) {
     int nch = (ncells + chunk_cells - 1) / chunk_cells;
     // All chunks of a chain sit in shared memory together.  A model whose chain does not fit (M >= 3072) gets no tiles:
     // every pair of it goes straight to the exact MSV kernel (ssv_bypass_kernel), which has no such limit.
-    if ((int64_t)nch * tile_block_bytes_host(chainJ) > cap) { db.ssv_bypass.push_back(it.model); continue; }
+    if ((int64_t)nch * ssv_block_bytes(chainJ, tmem) > cap) { db.ssv_bypass.push_back(it.model); continue; }
     chains.push_back({(int)tiles.size(), nch});
     for (int c = 0; c < nch; ++c) {
       HostTile ht{chainJ, {}, 64, c > 0, c + 1 < nch};
@@ -96,16 +97,17 @@ static void build_tiles(ckm_models &db, std::vector<uint8_t> &blob) {
     td.chain_next = tiles[t].chain_next; td.chain_prev = tiles[t].chain_prev; td.table_off = off;
     for (auto &tm : tiles[t].tm) db.tile_models.push_back(tm);
     db.tiles.push_back(td);
-    off += tile_block_bytes_host(td.J);
+    off += ssv_block_bytes(td.J, tmem);
   }
   blob.assign((size_t)off, 0);
   {
     TileGroup g{}; bool open = false; int64_t gbytes = 0;
     for (size_t c = 0; c < chains.size(); ++c) {
       int t0 = chains[c].first, nt = chains[c].second, J = tiles[t0].J;
-      int64_t need = (int64_t)nt * tile_block_bytes_host(J);
+      int64_t need = (int64_t)nt * ssv_block_bytes(J, tmem);
       if (need > cap) throw std::runtime_error("model " + db.models[tiles[t0].tm[0].model].name + " is too long for the SSV tiles");
-      if (open && (g.J != J || gbytes + need > cap)) { g.table_bytes = gbytes; db.groups.push_back(g); open = false; }
+      // a TMEM-assisted tile is alone in its group: tensor memory holds the words of one tile
+      if (open && (g.J != J || gbytes + need > cap || (tmem && J == 32))) { g.table_bytes = gbytes; db.groups.push_back(g); open = false; }
       if (!open) { g = TileGroup{}; g.J = J; g.first_tile = t0; g.ntiles = 0; g.nchains = 0; g.first_chain = (int)c; g.table_off = db.tiles[t0].table_off; gbytes = 0; open = true; }
       g.ntiles += nt; g.nchains += 1; gbytes += need;
       db.chain_first_tile.push_back(t0); db.chain_ntiles.push_back(nt);
@@ -116,11 +118,11 @@ static void build_tiles(ckm_models &db, std::vector<uint8_t> &blob) {
   for (size_t t = 0; t < tiles.size(); ++t) {
     const int J = tiles[t].J;
     uint8_t *base = blob.data() + db.tiles[t].table_off;
-    const bool i8 = (J == 32);
-    const int RB = ssv_row_bytes(J);
-    float *A = reinterpret_cast<float *>(base + ssv_table_bytes(J));
-    int32_t *F = reinterpret_cast<int32_t *>(base + ssv_table_bytes(J) + 256);
-    int32_t *SM = reinterpret_cast<int32_t *>(base + ssv_table_bytes(J) + 512);
+    const bool i8 = ssv_int8_chunk(J, tmem);
+    const int RB = ssv_row_bytes(J, tmem);
+    float *A = reinterpret_cast<float *>(base + ssv_table_bytes(J, tmem));
+    int32_t *F = reinterpret_cast<int32_t *>(base + ssv_table_bytes(J, tmem) + 256);
+    int32_t *SM = reinterpret_cast<int32_t *>(base + ssv_table_bytes(J, tmem) + 512);
     for (int s = 0; s < 64; ++s) { A[s] = 1e30f; F[s] = 1 << 28; SM[s] = -1; }
     // where the gain of cell (lane, half, q) for residue x lives, and a store that knows the cell's width
     auto put = [&](int x, int lane, int half, int q, int d) {
@@ -156,8 +158,8 @@ static void build_tiles(ckm_models &db, std::vector<uint8_t> &blob) {
   for (size_t t = 0; t < tiles.size(); ++t) {
     const int J = tiles[t].J;
     uint8_t *base = blob.data() + db.tiles[t].table_off;
-    float *A = reinterpret_cast<float *>(base + ssv_table_bytes(J));
-    int32_t *F = reinterpret_cast<int32_t *>(base + ssv_table_bytes(J) + 256);
+    float *A = reinterpret_cast<float *>(base + ssv_table_bytes(J, tmem));
+    int32_t *F = reinterpret_cast<int32_t *>(base + ssv_table_bytes(J, tmem) + 256);
     for (auto &tm : tiles[t].tm) {
       const Model &m = db.models[tm.model];
       const double F1 = 0.02;

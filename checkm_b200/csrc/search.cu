@@ -151,7 +151,7 @@ static int run_stage1(ckm_engine *e, const ckm_models *m, const ckm_seqdb *db, A
     for (int g : gl[c]) maxbytes = std::max<int64_t>(maxbytes, m->groups[g].table_bytes);
     const int64_t units = (int64_t)p.ngroups * p.nchunks;
     const int grid = (int)std::min<int64_t>(nsm, units);
-    if ((rc = launch_ssv(Js[c], p, grid, (size_t)maxbytes, st))) return rc;
+    if ((rc = launch_ssv(Js[c], m->ssv_tmem, p, grid, (size_t)maxbytes, st))) return rc;
     e->stats.kernel_launches++;
   }
   if (!m->ssv_bypass.empty()) {

@@ -38,7 +38,7 @@ struct SsvParams {
   double F1;
 };
 
-int launch_ssv(int J, const SsvParams &p, int grid, size_t smem_bytes, cudaStream_t stream);
+int launch_ssv(int J, bool tmem, const SsvParams &p, int grid, size_t smem_bytes, cudaStream_t stream);   // tmem: J = 32 tiles in the TMEM-assisted layout
 
 // ---- stage 1b: exact MSV on the candidates ----
 struct MsvParams {
